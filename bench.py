@@ -63,7 +63,31 @@ def parse():
     ap.add_argument("--recordings", type=int, default=10)
     ap.add_argument("--recording-seconds", type=int, default=600)
     ap.add_argument("--ref-clips", type=int, default=0, help="--impl reference: clips per step (0 = sized from K + W)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the timed path returned in its last step (token ids and lengths of "
+                         "rank 0) as DIR/<name>.npy, float32; inputs and weights are seeded, so two builds compare output for output")
     return ap.parse_args()
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT_BYTES):
+    """Writes `arrays` (name -> array, one row per clip or window) as <out_dir>/<name>.npy in float32, which holds every token
+    id and length exactly.  When the files would exceed `limit` bytes in all, the same fixed seeded sample of rows is kept in
+    every array and the row indices are written as rows.npy (float64)."""
+    import numpy as np
+    arrays = {k: np.asarray(v, dtype=np.float32) for k, v in arrays.items()}
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a.nbytes for a in arrays.values()) // max(n, 1)
+    budget = limit - 4096           # room for the .npy headers
+    if n * row_bytes > budget:
+        rows = np.sort(np.random.default_rng(0).choice(n, size=budget // (row_bytes + 8), replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), a)
 
 
 class ClockSampler:
@@ -193,15 +217,16 @@ def run_reference(args, rank, world):
     def step(i):
         x = pcm[i * clips_per_step:(i + 1) * clips_per_step]
         feats = hf_ref.hf_features(fe, x)
-        ids = hf_ref.hf_generate(model, feats, args.max_length, return_timestamps=False)
-        return ids.shape[1]
+        return hf_ref.hf_generate(model, feats, args.max_length, return_timestamps=False)
 
     for i in range(args.warmup):
         step(i)
     t0 = time.perf_counter()
     for i in range(args.steps):
-        step(args.warmup + i)
+        ids = step(args.warmup + i)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"tokens": ids})
     v = clips_per_step * args.steps * CLIP_SECONDS / dt
     sample = (f"{clips_per_step} clips per step (one HF batch) of the {args.batch}-clip batch, full max_length={args.max_length}, "
               f"fp32, {cores} threads")
@@ -404,9 +429,11 @@ def run_longform(args, rank, world, local_rank):
     e0.record()
     for _ in range(K):
         f, st = windows(recs_dev)
-        decode_all(f)
+        last = decode_all(f)
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"tokens": last[0].cpu(), "lengths": last[1].cpu()})
     ms = e0.elapsed_time(e1)
     launches = model.ctx.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
@@ -554,6 +581,7 @@ def main():
                                                model._rules(False)["pad"], world * K * B)
     e1.record()
     barrier()
+    last_out = outs[-1]          # what the headline's timed path returned in its last step (replaced when the pipeline runs)
     ms = e0.elapsed_time(e1)
     launches = model.ctx.launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
@@ -660,6 +688,7 @@ def main():
             if rank == 0:
                 sampler.start()
             p_ms, p_launches, got = timed_pipeline(lambda i: dev_batches[i % len(dev_batches)])
+            last_out = (torch.cat([g[0] for g in got[-G:]]), torch.cat([g[1] for g in got[-G:]]))
             clocks = sampler.stop() if rank == 0 else None
             if world > 1:       # final result gather (the only collective of the path)
                 from taiwan_whisper_b200.shard import gather_token_rows
@@ -795,6 +824,8 @@ def main():
                     line["extra"] = hf_cuda_comparator(args, hf_cpu, host_batches[0], dev)
                 except Exception as e:
                     line["extra"] = {"hf_cuda_error": f"{type(e).__name__}: {e}"}
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, {"tokens": last_out[0].cpu(), "lengths": last_out[1].cpu()})
         print(json.dumps(line))
     if world > 1:
         dist.barrier()
