@@ -258,6 +258,39 @@ TW_API int tw_debug_self_attention(tw_ctx* ctx, const void* q, int64_t q_stride,
 TW_API int tw_debug_encoder_attention(tw_ctx* ctx, const void* qkv, void* out, int B, int S, int H, int dtype, int impl,
                                       void* stream);
 
+/* Test entry points for the kernels of one decode step in the form the step issues them: state on the device (position, finished
+ * flags, active-clip list, page table) and the SM count of the partition the step runs in.  Device buffers unless noted.
+ *
+ * tw_debug_select_steps: the greedy loop of tw_decode_greedy (same decode state, step header, rules upload and per-row budgets) with
+ *   caller-supplied logits in place of the model forward.  logits float32 [max_length - P, B, ld_logits] (16-byte aligned, ld_logits
+ *   >= vocab and a multiple of 4): scores of generated step g at logits + g*B*ld_logits; columns >= vocab are never selected.
+ *   prompt / rules (host), forced, logits_tap, tap_steps, out_tokens [B, max_length - P], out_lengths [B]: as tw_decode_greedy.
+ *   row_budgets (host int32 [B], nullable): the budgets of tw_debug_set_row_budgets for this call only (they are off afterwards);
+ *   NULL leaves the budgets set with tw_debug_set_row_budgets in effect.  n_active [max_length - P] and active
+ *   [max_length - P, B] (nullable): the active-clip count and list after every generated step.
+ * tw_debug_kv_append: the self-attention QKV projection C [M, 3d] = A [M, d] . W [3d, d]^T + bias of a decode step at position *d_pos,
+ *   whose K|V columns land in pool row page_table[m * pt_stride + pos / 16] * 16 + pos % 16 (pool [n_pages][16][2d]).
+ *   fused = 1 (bf16, M <= 256): one skinny GEMM that stores columns >= d in the pool instead of C (C[:, d:] is not written);
+ *   fused = 0: the GEMM into C, then the append kernel (bf16 or fp32).  n_sms > 0 sizes the GEMM for a partition of that many SMs.
+ * tw_debug_self_attention_step: decoder self-attention with Tk = *d_pos + 1 rows per clip read on the device (old rows are fetched
+ *   before the programmatic-dependency wait); kv / page_table as tw_debug_self_attention(_paged) (page_table NULL: contiguous rows,
+ *   clip stride kv_clip_stride).  finished (int32 [B], nullable): rows whose flag is set are not computed and their out rows are left
+ *   as they were.  variant: 0 the build's default kernel, 1 registers, 2 shared-memory ring.
+ * tw_debug_decode_attention_step: the cross-attention K|V stream of tw_debug_decode_attention over the compacted active-clip list
+ *   (active int32 [B], n_active int32 [1], both NULL = every clip): only clips active[0 .. *n_active) are computed, other out rows
+ *   are left as they were.  n_sms > 0: the stream runs as in a pipeline partition of that many SMs. */
+TW_API int tw_debug_select_steps(tw_model* m, const float* logits, int64_t ld_logits, int B, const int32_t* prompt, int P,
+                                 const tw_rules* rules, int max_length, const int32_t* row_budgets, const int32_t* forced, float* logits_tap,
+                                 int tap_steps, int32_t* out_tokens, int32_t* out_lengths, int32_t* n_active, int32_t* active, void* stream);
+TW_API int tw_debug_kv_append(tw_ctx* ctx, const void* A, const void* W, const float* bias, void* C, void* pool, const int32_t* page_table,
+                              int pt_stride, const int32_t* d_pos, int M, int d, int dtype, int fused, int n_sms, void* stream);
+TW_API int tw_debug_self_attention_step(tw_ctx* ctx, const void* q, int64_t q_stride, const void* kv, int64_t kv_clip_stride,
+                                        const int32_t* page_table, int pt_stride, const int32_t* d_pos, const int32_t* finished, int B, int H,
+                                        int dtype, int variant, void* out, void* stream);
+TW_API int tw_debug_decode_attention_step(tw_ctx* ctx, const void* q, int64_t q_stride, const void* kv, int64_t kv_clip_stride, int Tk,
+                                          int B, int H, int dtype, const int32_t* active, const int32_t* n_active, int n_sms, void* out,
+                                          void* stream);
+
 #ifdef __cplusplus
 }
 #endif

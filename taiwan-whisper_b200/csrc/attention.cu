@@ -788,14 +788,14 @@ self_attention_decode_ring_kernel(const T* __restrict__ q, int64_t q_stride, con
 
 template <typename T>
 void self_attention_decode(const T* q, int64_t q_stride, const T* kv, int64_t kv_clip_stride, int Tk, const int32_t* d_tk, int B, int H,
-                           T* out, cudaStream_t st, const int32_t* page_table, int pt_stride, const int32_t* finished) {
+                           T* out, cudaStream_t st, const int32_t* page_table, int pt_stride, const int32_t* finished, int variant) {
     dim3 grid(ceil_div(H, SA_HG), B);
     // early: old cache rows are fetched before the programmatic-dependency wait (only inside the decode step, where the row count
     // comes from the device-side position and rows below it are older than the previous kernel); TWB200_SA_EARLY=0 switches it off
     static const bool early_on = !(getenv("TWB200_SA_EARLY") && atoi(getenv("TWB200_SA_EARLY")) == 0);
     // ring variant (cp.async into shared memory, 8 rows in flight per warp all the time): bf16 default; TWB200_SA_RING=0 / 1 forces
     static const int ring_env = getenv("TWB200_SA_RING") ? atoi(getenv("TWB200_SA_RING")) : -1;
-    const bool ring = ring_env >= 0 ? ring_env != 0 : sizeof(T) == 2;
+    const bool ring = variant == SA_VARIANT_RING || (variant == SA_VARIANT_DEFAULT && (ring_env >= 0 ? ring_env != 0 : sizeof(T) == 2));
     if (ring) {
         constexpr int smem = SA_WARPS * SA_RING * 2 * 32 * 8 * (int)sizeof(T);
         static bool attr_set = false;
@@ -811,9 +811,9 @@ void self_attention_decode(const T* q, int64_t q_stride, const T* kv, int64_t kv
              page_table, pt_stride, finished, (early_on && d_tk) ? 1 : 0);
 }
 template void self_attention_decode<float>(const float*, int64_t, const float*, int64_t, int, const int32_t*, int, int, float*,
-                                           cudaStream_t, const int32_t*, int, const int32_t*);
+                                           cudaStream_t, const int32_t*, int, const int32_t*, int);
 template void self_attention_decode<__nv_bfloat16>(const __nv_bfloat16*, int64_t, const __nv_bfloat16*, int64_t, int, const int32_t*,
-                                                   int, int, __nv_bfloat16*, cudaStream_t, const int32_t*, int, const int32_t*);
+                                                   int, int, __nv_bfloat16*, cudaStream_t, const int32_t*, int, const int32_t*, int);
 
 static int g_da_sm_dev = 0;       // SMs of the device: sizes the partial-record workspace
 static int g_da_sm_count = 0;     // CTAs of the stream kernel = SMs the launching stream may use (decode_attention_set_sms)
@@ -827,9 +827,11 @@ size_t decode_attention_partial_floats(int B, int H) {
     }
     return (size_t)(g_da_sm_dev + B) * H * DA_PSTRIDE;
 }
-void decode_attention_set_sms(int n) {
+int decode_attention_set_sms(int n) {
     (void)decode_attention_partial_floats(1, 1);
+    const int prev = g_da_sm_count;
     g_da_sm_count = (n > 0 && n < g_da_sm_dev) ? n : g_da_sm_dev;
+    return prev;
 }
 
 template <typename T>

@@ -121,13 +121,17 @@ void decode_attention(const T* q, int64_t q_stride, const T* kv, int64_t kv_clip
                       float* partial, T* out, cudaStream_t st, cudaEvent_t ev0 = nullptr, cudaEvent_t ev1 = nullptr,
                       const int32_t* active = nullptr, const int32_t* n_active = nullptr);
 size_t decode_attention_partial_floats(int B, int H);
-// the K|V stream kernel launches one CTA per SM: n = SMs of the partition its stream runs in (0 = the whole device)
-void decode_attention_set_sms(int n);
-// single-launch self-attention over the short decoder cache (Tk = *d_tk + 1 when d_tk is given)
+// the K|V stream kernel launches one CTA per SM: n = SMs of the partition its stream runs in (0 = the whole device); returns the
+// previous count
+int decode_attention_set_sms(int n);
+// single-launch self-attention over the short decoder cache (Tk = *d_tk + 1 when d_tk is given).  Two kernels with the same row
+// order and arithmetic: registers (4 rows in flight per warp) and a cp.async shared-memory ring (8 rows); SA_VARIANT_DEFAULT takes
+// the ring for bf16 and the register kernel for fp32 (TWB200_SA_RING=0 / 1 overrides that default for the process).
+enum { SA_VARIANT_DEFAULT = 0, SA_VARIANT_REGISTER = 1, SA_VARIANT_RING = 2 };
 template <typename T>
 void self_attention_decode(const T* q, int64_t q_stride, const T* kv, int64_t kv_clip_stride, int Tk, const int32_t* d_tk, int B, int H,
                            T* out, cudaStream_t st, const int32_t* page_table = nullptr, int pt_stride = 0,
-                           const int32_t* finished = nullptr);
+                           const int32_t* finished = nullptr, int variant = SA_VARIANT_DEFAULT);
 
 // ---- absorbed cross-attention (absorb.cu), bf16 only: scores and values straight from the encoder output through per-head
 // q~ = Wk_h^T q_h; returns c_h = softmax(q~_h . E^T) E per clip and head.  qt [B*H + ABSORB_QT_PAD rows, d] (row clip*H + h),

@@ -723,17 +723,17 @@ int launch_step(tw_model* m, int B, const RulesDev& R, const DecodeState& S, con
     return TW_OK;
 }
 
-template <typename T>
-int decode_impl(tw_model* m, int B, const int32_t* prompt, int P, const RulesDev& R, int max_length, int32_t* out_tokens,
-                int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps, cudaStream_t st) {
+// Decode state of one call (the model's dstate arrays, initialised for B rows), the cleared out_lengths and the step header
+// (position 0, prompt, output stride, tapped steps) on the device: shared by decode_impl and tw_debug_select_steps.
+int begin_decode(tw_model* m, int B, const int32_t* prompt, int P, int max_length, int32_t* out_lengths, float* logits_tap, int tap_steps,
+                 cudaStream_t st, DecodeState* out) {
     const tw_model_desc& D = m->desc;
     tw_ctx* ctx = m->ctx;
-    const int n_gen_max = max_length - P;
     if (P > STEP_INTS - STEP_PROMPT) {
         ctx->set_error(TW_E_INVALID, "decode: prompt longer than 24 tokens is not supported");
         return TW_E_INVALID;
     }
-    DecodeState S;
+    DecodeState& S = *out;
     S.cur_tok = m->dstate;
     S.finished = m->dstate + D.max_batch;
     S.n_gen = m->dstate + 2 * D.max_batch;
@@ -750,10 +750,20 @@ int decode_impl(tw_model* m, int B, const int32_t* prompt, int P, const RulesDev
     int32_t* hs = m->h_step;
     TW_CUDA_OK(ctx, cudaStreamSynchronize(st));          // previous call may still be reading h_step
     for (int i = 0; i < STEP_INTS; ++i) hs[i] = 0;
-    hs[STEP_POS] = 0; hs[STEP_P] = P; hs[STEP_STRIDE] = n_gen_max; hs[STEP_TAP] = logits_tap ? tap_steps : 0;
+    hs[STEP_POS] = 0; hs[STEP_P] = P; hs[STEP_STRIDE] = max_length - P; hs[STEP_TAP] = logits_tap ? tap_steps : 0;
     for (int i = 0; i < P; ++i) hs[STEP_PROMPT + i] = prompt[i];
     TW_CUDA_OK(ctx, cudaMemcpyAsync(m->d_step, hs, STEP_INTS * sizeof(int32_t), cudaMemcpyHostToDevice, st));
     ctx->launches += 1;
+    return TW_OK;
+}
+
+template <typename T>
+int decode_impl(tw_model* m, int B, const int32_t* prompt, int P, const RulesDev& R, int max_length, int32_t* out_tokens,
+                int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps, cudaStream_t st) {
+    tw_ctx* ctx = m->ctx;
+    const int n_gen_max = max_length - P;
+    DecodeState S;
+    TW_CHECK(begin_decode(m, B, prompt, P, max_length, out_lengths, logits_tap, tap_steps, st, &S));
     // page table of this call: only the ceil(max_length / TW_KV_PAGE) pages a clip can reach are mapped, page-major
     // (logical page p of clip b -> physical page p*B + b), so a call touches a dense prefix of every layer's pool whose
     // size follows B and max_length, and the B cache rows written by one step are adjacent
@@ -1499,23 +1509,32 @@ int tw_debug_gemm(tw_ctx* ctx, const void* A, const void* W, const float* bias, 
     return TW_OK;
 }
 
+}  // extern "C"
+
+namespace {
+// partial-record workspace of the tw_debug_* K|V stream launches: one allocation for every shape they accept (B <= 4096, H <= 20),
+// zeroed when the call shape changes (it holds the arrival counters)
+int debug_da_scratch(tw_ctx* ctx, int B, int H, float** out) {
+    static float* scratch = nullptr;
+    static int scratch_B = -1, scratch_H = -1;
+    const size_t floats = decode_attention_partial_floats(4096, 20);
+    if (!scratch) TW_CUDA_OK(ctx, cudaMalloc(&scratch, floats * sizeof(float)));
+    if (B != scratch_B || H != scratch_H) {
+        TW_CUDA_OK(ctx, cudaMemset(scratch, 0, floats * sizeof(float)));
+        scratch_B = B; scratch_H = H;
+    }
+    *out = scratch;
+    return TW_OK;
+}
+}  // namespace
+
+extern "C" {
+
 int tw_debug_decode_attention(tw_ctx* ctx, const void* q, int64_t q_stride, const void* kv, int64_t kv_clip_stride, int Tk, int B,
                               int H, int dtype, void* out, void* stream) {
     if (!ctx || !q || !kv || !out || B <= 0 || B > 4096 || Tk <= 0 || H <= 0 || H > 20) return TW_E_INVALID;
-    // scratch sized (and zeroed: it holds the arrival counters) per call shape
-    static float* scratch = nullptr;
-    static size_t scratch_floats = 0;
-    static int scratch_B = -1, scratch_H = -1;
-    const size_t need = decode_attention_partial_floats(B, H);
-    if (need > scratch_floats || B != scratch_B || H != scratch_H) {
-        if (need > scratch_floats) {
-            if (scratch) cudaFree(scratch);
-            TW_CUDA_OK(ctx, cudaMalloc(&scratch, need * sizeof(float)));
-            scratch_floats = need;
-        }
-        TW_CUDA_OK(ctx, cudaMemset(scratch, 0, scratch_floats * sizeof(float)));
-        scratch_B = B; scratch_H = H;
-    }
+    float* scratch = nullptr;
+    TW_CHECK(debug_da_scratch(ctx, B, H, &scratch));
     cudaStream_t st = (cudaStream_t)stream;
     if (dtype == TW_BF16)
         decode_attention<__nv_bfloat16>((const __nv_bfloat16*)q, q_stride, (const __nv_bfloat16*)kv, kv_clip_stride, Tk, nullptr, B, H,
@@ -1555,6 +1574,92 @@ int tw_debug_self_attention_paged(tw_ctx* ctx, const void* q, int64_t q_stride, 
     ctx->launches += 1;
     TW_CUDA_OK(ctx, cudaGetLastError());
     return TW_OK;
+}
+
+int tw_debug_decode_attention_step(tw_ctx* ctx, const void* q, int64_t q_stride, const void* kv, int64_t kv_clip_stride, int Tk, int B,
+                                   int H, int dtype, const int32_t* active, const int32_t* n_active, int n_sms, void* out, void* stream) {
+    if (!ctx || !q || !kv || !out || B <= 0 || B > 4096 || Tk <= 0 || H <= 0 || H > 20 || (!active) != (!n_active) ||
+        (dtype != TW_BF16 && dtype != TW_F32))
+        return TW_E_INVALID;
+    float* scratch = nullptr;
+    TW_CHECK(debug_da_scratch(ctx, B, H, &scratch));
+    cudaStream_t st = (cudaStream_t)stream;
+    // the grid of the stream kernel and the partition's SM count, as set_active_sms sets them for a pipeline stage
+    const int sms_before = ctx->sm_count;
+    const int da_before = decode_attention_set_sms(n_sms > 0 ? n_sms : 0);
+    if (n_sms > 0) ctx->sm_count = n_sms;
+    if (dtype == TW_BF16)
+        decode_attention<__nv_bfloat16>((const __nv_bfloat16*)q, q_stride, (const __nv_bfloat16*)kv, kv_clip_stride, Tk, nullptr, B, H,
+                                        scratch, (__nv_bfloat16*)out, st, nullptr, nullptr, active, n_active);
+    else
+        decode_attention<float>((const float*)q, q_stride, (const float*)kv, kv_clip_stride, Tk, nullptr, B, H, scratch, (float*)out, st,
+                                nullptr, nullptr, active, n_active);
+    decode_attention_set_sms(da_before);
+    ctx->sm_count = sms_before;
+    ctx->launches += 2;
+    TW_CUDA_OK(ctx, cudaGetLastError());
+    return TW_OK;
+}
+
+int tw_debug_self_attention_step(tw_ctx* ctx, const void* q, int64_t q_stride, const void* kv, int64_t kv_clip_stride, const int32_t* page_table,
+                                 int pt_stride, const int32_t* d_pos, const int32_t* finished, int B, int H, int dtype, int variant, void* out,
+                                 void* stream) {
+    if (!ctx || !q || !kv || !d_pos || !out || B <= 0 || H <= 0 || (page_table && pt_stride <= 0) || variant < SA_VARIANT_DEFAULT ||
+        variant > SA_VARIANT_RING || (dtype != TW_BF16 && dtype != TW_F32))
+        return TW_E_INVALID;
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == TW_BF16)
+        self_attention_decode<__nv_bfloat16>((const __nv_bfloat16*)q, q_stride, (const __nv_bfloat16*)kv, kv_clip_stride, 0, d_pos, B, H,
+                                             (__nv_bfloat16*)out, st, page_table, pt_stride, finished, variant);
+    else
+        self_attention_decode<float>((const float*)q, q_stride, (const float*)kv, kv_clip_stride, 0, d_pos, B, H, (float*)out, st, page_table,
+                                     pt_stride, finished, variant);
+    ctx->launches += 1;
+    TW_CUDA_OK(ctx, cudaGetLastError());
+    return TW_OK;
+}
+
+int tw_debug_kv_append(tw_ctx* ctx, const void* A, const void* W, const float* bias, void* C, void* pool, const int32_t* page_table,
+                       int pt_stride, const int32_t* d_pos, int M, int d, int dtype, int fused, int n_sms, void* stream) {
+    if (!ctx || !A || !W || !C || !pool || !page_table || !d_pos || M <= 0 || d <= 0 || pt_stride <= 0 ||
+        (dtype != TW_BF16 && dtype != TW_F32) || (fused && dtype != TW_BF16))
+        return TW_E_INVALID;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int sms_before = ctx->sm_count;
+    if (n_sms > 0) ctx->sm_count = n_sms;          // the skinny GEMM sizes its tiles and grid from it
+    GemmEpi e = mk_epi(EPI_STORE, bias, C, 3 * d);
+    int r = TW_OK;
+    if (dtype == TW_BF16) {
+        typedef __nv_bfloat16 T;
+        const bool skinny = gemm_tc_skinny_supported(M, 3 * d, d, e);
+        if (fused) {
+            // as launch_step issues it: the K|V columns go to the pool row of (row, *d_pos) through the page table
+            e.n_split = d;
+            e.C2 = pool;
+            e.ldc2 = 0;
+            e.d_row2 = d_pos;
+            e.row2_stride = 2 * d;
+            e.page_table = page_table;
+            e.pt_stride = pt_stride;
+            if (!skinny) {
+                ctx->set_error(TW_E_UNSUPPORTED, "tw_debug_kv_append: the fused append needs the skinny GEMM (M <= 256, d % 64 == 0)");
+                r = TW_E_UNSUPPORTED;
+            } else {
+                r = gemm_tc_skinny(ctx, (const T*)A, d, (const T*)W, d, M, 3 * d, d, e, st);
+            }
+        } else {
+            r = skinny ? gemm_tc_skinny(ctx, (const T*)A, d, (const T*)W, d, M, 3 * d, d, e, st)
+                       : gemm_tc(ctx, (const T*)A, d, (const T*)W, d, M, 3 * d, d, e, st);
+            if (r == TW_OK) kv_append<T>((const T*)C, (T*)pool, d_pos, M, d, 0, st, page_table, pt_stride);
+        }
+    } else {
+        gemm_simt<float>((const float*)A, d, (const float*)W, d, M, 3 * d, d, e, st);
+        kv_append<float>((const float*)C, (float*)pool, d_pos, M, d, 0, st, page_table, pt_stride);
+    }
+    ctx->sm_count = sms_before;
+    ctx->launches += fused ? 1 : 2;
+    if (r == TW_OK) TW_CUDA_OK(ctx, cudaGetLastError());
+    return r;
 }
 
 int tw_debug_encoder_attention(tw_ctx* ctx, const void* qkv, void* out, int B, int S, int H, int dtype, int impl, void* stream) {
@@ -1602,6 +1707,45 @@ int tw_debug_set_row_budgets(tw_model* m, const int32_t* budgets_host, int n) {
         TW_CUDA_OK(m->ctx, cudaMemcpy(m->d_row_budget, tmp.data(), tmp.size() * sizeof(int32_t), cudaMemcpyHostToDevice));
     }
     return TW_OK;
+}
+
+int tw_debug_select_steps(tw_model* m, const float* logits, int64_t ld_logits, int B, const int32_t* prompt, int P, const tw_rules* rules,
+                          int max_length, const int32_t* row_budgets, const int32_t* forced, float* logits_tap, int tap_steps,
+                          int32_t* out_tokens, int32_t* out_lengths, int32_t* n_active, int32_t* active, void* stream) {
+    if (!check_model(m, "tw_debug_select_steps")) return TW_E_INVALID;
+    TW_CHECK(check_decode_args(m, B, prompt, P, rules, max_length));
+    tw_ctx* ctx = m->ctx;
+    const int V = m->desc.vocab, n_gen = max_length - P;
+    if (!logits || !out_tokens || !out_lengths || ld_logits < V || (ld_logits % 4) || (reinterpret_cast<uintptr_t>(logits) & 15) ||
+        (logits_tap && (tap_steps < 0 || tap_steps > n_gen))) {
+        ctx->set_error(TW_E_INVALID, "tw_debug_select_steps: null buffer, or logits without a 16-byte aligned base and a row pitch >= vocab "
+                                     "that is a multiple of 4 floats, or tap_steps outside 0 .. max_length - P");
+        return TW_E_INVALID;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    RulesDev R;
+    TW_CHECK(upload_rules(m, rules, &R, st));
+    const bool budgets_before = m->row_budget_on;
+    TW_CHECK(tw_debug_set_row_budgets(m, row_budgets, row_budgets ? B : 0));
+    DecodeState S;
+    int r = begin_decode(m, B, prompt, P, max_length, out_lengths, logits_tap, tap_steps, st, &S);
+    // the decode loop of decode_impl with the logits of generated step g read from logits + g * B * ld_logits instead of the model
+    for (int pos = 0; r == TW_OK && pos < max_length - 1; ++pos) {
+        const int g = pos - (P - 1);
+        select_tokens(logits + (int64_t)(g > 0 ? g : 0) * B * ld_logits, ld_logits, V, B, m->d_step, R, S, out_tokens, out_lengths, forced,
+                      logits_tap, st);
+        advance_step(m->d_step, S, B, st);
+        ctx->launches += 2;
+        if (g >= 0 && n_active && cudaMemcpyAsync(n_active + g, S.n_active, sizeof(int32_t), cudaMemcpyDeviceToDevice, st) != cudaSuccess) r = TW_E_CUDA;
+        if (g >= 0 && active && cudaMemcpyAsync(active + (int64_t)g * B, S.active, B * sizeof(int32_t), cudaMemcpyDeviceToDevice, st) != cudaSuccess)
+            r = TW_E_CUDA;
+    }
+    // budgets given here apply to this call only; without them the budgets of tw_debug_set_row_budgets stay as they were
+    if (row_budgets) m->row_budget_on = false;
+    else m->row_budget_on = budgets_before;
+    if (r == TW_E_CUDA) ctx->set_error(TW_E_CUDA, std::string("tw_debug_select_steps: ") + cudaGetErrorString(cudaGetLastError()));
+    if (r == TW_OK) TW_CUDA_OK(ctx, cudaGetLastError());
+    return r;
 }
 
 int tw_profile(tw_model* m, int enable, float* total_ms, int* launches, double* bytes_per_launch) {
