@@ -291,6 +291,22 @@ TW_API int tw_debug_decode_attention_step(tw_ctx* ctx, const void* q, int64_t q_
                                           int B, int H, int dtype, const int32_t* active, const int32_t* n_active, int n_sms, void* out,
                                           void* stream);
 
+/* Test entry points for the encoder stage (stage 1: encoder + cross-attention K|V store) in the form the model issues it.
+ * tw_debug_layernorm: out [M, d] (dtype TW_F32 / TW_BF16) = LayerNorm of the float32 rows x [M, d] with float32 gamma / beta [d],
+ *   through the launcher the model uses, so M picks the kernel as in the model (one CTA per row for M <= 512, one warp per row
+ *   above).  TW_E_INVALID for M < 0, d > 1280, d % 4 != 0, another dtype or a null buffer; M = 0 launches nothing.
+ * tw_debug_cross_kv: the cross-attention K|V projection of every decoder layer for clips clip0 .. clip0 + B - 1 into the model's
+ *   own K|V store (the one tw_decode_greedy reads; with the pipeline on, slot 0's), from enc_out [B, 1500, d_model] in the model
+ *   dtype.  Rows of other clips are not written.
+ * tw_debug_read_stage1: copies (cudaMemcpyAsync on `stream`) the rows of clips clip0 .. clip0 + B - 1: the encoder output of pipeline
+ *   slot 0 / 1 into enc_out [B, 1500, d_model] (nullable; must be NULL for slot -1) and decoder layer `layer`'s K|V rows into kv_out
+ *   [B, 1500, 2 d_model] (nullable), from the slot's store or, for slot -1, from the model's own store.  For slots 0 / 1 the copies
+ *   first wait for the slot's last tw_pipeline_encode(_at). */
+TW_API int tw_debug_layernorm(tw_ctx* ctx, const float* x, const float* gamma, const float* beta, void* out, int M, int d, int dtype,
+                              void* stream);
+TW_API int tw_debug_cross_kv(tw_model* m, const void* enc_out, int B, int clip0, void* stream);
+TW_API int tw_debug_read_stage1(tw_model* m, int slot, int clip0, int B, void* enc_out, int layer, void* kv_out, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

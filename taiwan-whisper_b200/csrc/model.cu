@@ -1509,6 +1509,56 @@ int tw_debug_gemm(tw_ctx* ctx, const void* A, const void* W, const float* bias, 
     return TW_OK;
 }
 
+int tw_debug_layernorm(tw_ctx* ctx, const float* x, const float* gamma, const float* beta, void* out, int M, int d, int dtype,
+                       void* stream) {
+    if (!ctx) return TW_E_INVALID;
+    if (!x || !gamma || !beta || !out || M < 0 || d <= 0 || d > 1280 || d % 4 || (dtype != TW_F32 && dtype != TW_BF16)) {
+        ctx->set_error(TW_E_INVALID, "tw_debug_layernorm: need M >= 0, 0 < d <= 1280 with d % 4 == 0, dtype float32 / bfloat16 and non-null buffers");
+        return TW_E_INVALID;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == TW_F32) layernorm<float>(x, gamma, beta, (float*)out, M, d, st);
+    else layernorm<__nv_bfloat16>(x, gamma, beta, (__nv_bfloat16*)out, M, d, st);
+    ctx->launches += 1;
+    TW_CUDA_OK(ctx, cudaGetLastError());
+    return TW_OK;
+}
+
+int tw_debug_cross_kv(tw_model* m, const void* enc_out, int B, int clip0, void* stream) {
+    if (!check_model(m, "tw_debug_cross_kv")) return TW_E_INVALID;
+    if (!enc_out || B <= 0 || clip0 < 0 || clip0 + B > m->desc.max_batch) {
+        m->ctx->set_error(TW_E_INVALID, "tw_debug_cross_kv: need 1 <= B, 0 <= clip0, clip0 + B <= max_batch and an encoder output");
+        return TW_E_INVALID;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    return m->desc.dtype == TW_BF16 ? cross_kv_impl<__nv_bfloat16>(m, enc_out, B, st, clip0) : cross_kv_impl<float>(m, enc_out, B, st, clip0);
+}
+
+int tw_debug_read_stage1(tw_model* m, int slot, int clip0, int B, void* enc_out, int layer, void* kv_out, void* stream) {
+    if (!check_model(m, "tw_debug_read_stage1")) return TW_E_INVALID;
+    tw_ctx* ctx = m->ctx;
+    const tw_model_desc& D = m->desc;
+    auto& P = m->pipe;
+    if (slot < -1 || slot > 1 || (slot >= 0 && !P.on) || (slot < 0 && enc_out) || B <= 0 || clip0 < 0 || clip0 + B > D.max_batch ||
+        (kv_out && (layer < 0 || layer >= D.dec_layers))) {
+        ctx->set_error(TW_E_INVALID, "tw_debug_read_stage1: bad slot (-1, or 0 / 1 with the pipeline on; no encoder output for -1), clip range or layer");
+        return TW_E_INVALID;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    const size_t d = D.d_model, e = m->esz, rows = (size_t)B * TW_N_CTX;
+    if (slot >= 0) TW_CUDA_OK(ctx, cudaStreamWaitEvent(st, P.enc_done[slot], 0));
+    if (enc_out) {
+        const char* src = (const char*)P.enc_out[slot] + (size_t)clip0 * TW_N_CTX * d * e;
+        TW_CUDA_OK(ctx, cudaMemcpyAsync(enc_out, src, rows * d * e, cudaMemcpyDeviceToDevice, st));
+    }
+    if (kv_out) {
+        const char* store = (const char*)(slot >= 0 ? P.xkv[slot] : m->xkv);
+        const char* src = store + ((size_t)layer * D.max_batch + clip0) * TW_N_CTX * 2 * d * e;
+        TW_CUDA_OK(ctx, cudaMemcpyAsync(kv_out, src, rows * 2 * d * e, cudaMemcpyDeviceToDevice, st));
+    }
+    return TW_OK;
+}
+
 }  // extern "C"
 
 namespace {

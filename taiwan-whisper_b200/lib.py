@@ -21,6 +21,7 @@ EXPORTS = [
     "tw_debug_decode_attention", "tw_debug_encoder_attention", "tw_debug_self_attention", "tw_debug_gemm_grouped",
     "tw_debug_absorbed_attention", "tw_pipeline_enable", "tw_pipeline_resize", "tw_pipeline_info", "tw_pipeline_stage_ms", "tw_pipeline_encode", "tw_pipeline_encode_at", "tw_pipeline_decode",
     "tw_debug_select_steps", "tw_debug_kv_append", "tw_debug_self_attention_step", "tw_debug_decode_attention_step",
+    "tw_debug_layernorm", "tw_debug_cross_kv", "tw_debug_read_stage1",
 ]
 
 
@@ -98,6 +99,9 @@ def load_library() -> C.CDLL:
     lib.tw_debug_kv_append.argtypes = [vp, vp, vp, vp, vp, vp, vp, C.c_int, vp, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, vp]
     lib.tw_debug_self_attention_step.argtypes = [vp, vp, i64, vp, i64, vp, C.c_int, vp, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp]
     lib.tw_debug_decode_attention_step.argtypes = [vp, vp, i64, vp, i64, C.c_int, C.c_int, C.c_int, C.c_int, vp, vp, C.c_int, vp, vp]
+    lib.tw_debug_layernorm.argtypes = [vp, vp, vp, vp, vp, C.c_int, C.c_int, C.c_int, vp]
+    lib.tw_debug_cross_kv.argtypes = [vp, vp, C.c_int, C.c_int, vp]
+    lib.tw_debug_read_stage1.argtypes = [vp, C.c_int, C.c_int, C.c_int, vp, C.c_int, vp, vp]
     lib.tw_pipeline_enable.argtypes = [vp, C.c_int]
     lib.tw_pipeline_resize.argtypes = [vp, C.c_int]
     lib.tw_pipeline_stage_ms.argtypes = [vp, C.c_int, C.POINTER(C.c_float), C.POINTER(C.c_float)]

@@ -8,6 +8,31 @@ def weights_np(hf_model):
     return {k: v.detach().float().numpy() for k, v in hf_model.state_dict().items()}
 
 
+PERTURBED = "-perturbed"     # test-parameter suffix: the shape's model with perturb_hf_model applied
+
+
+def split_shape(name):
+    """"tiny" -> ("tiny", False); "tiny-perturbed" -> ("tiny", True)."""
+    return (name[:-len(PERTURBED)], True) if name.endswith(PERTURBED) else (name, False)
+
+
+def perturb_hf_model(hf_model, seed=4321):
+    """Gives an HF Whisper model non-trivial biases and LayerNorms, in place: every existing bias ~ N(0, 0.05), every LayerNorm
+    gamma ~ 1 + N(0, 0.1) and beta ~ N(0, 0.1), drawn tensor by tensor from one seeded generator, so every layer gets its own
+    values and a parameter routed to the wrong layer or projection changes the result.  HF's init leaves every bias at 0 and every
+    LayerNorm at (1, 0), where such a mistake is invisible.  Embeddings and positions are left alone (EOS keeps its zero row)."""
+    import torch
+    g = torch.Generator().manual_seed(seed)
+    with torch.no_grad():
+        for _, mod in hf_model.named_modules():
+            if isinstance(mod, torch.nn.LayerNorm):
+                mod.weight.copy_(1.0 + 0.1 * torch.randn(mod.weight.shape, generator=g))
+                mod.bias.copy_(0.1 * torch.randn(mod.bias.shape, generator=g))
+            elif isinstance(mod, (torch.nn.Linear, torch.nn.Conv1d)) and mod.bias is not None:
+                mod.bias.copy_(0.05 * torch.randn(mod.bias.shape, generator=g))
+    return hf_model
+
+
 def default_rules(vocab, timestamps=False, suppress=True):
     ids = token_ids(vocab)
     special = [ids.sot, ids.translate, ids.transcribe, ids.startofprev - 1, ids.startofprev, ids.nospeech]

@@ -13,14 +13,14 @@ import pytest
 import torch
 
 from taiwan_whisper_b200.configs import SHAPES, token_ids
-from tests.helpers import default_rules, prompt_ids, weights_np
+from tests.helpers import PERTURBED, default_rules, perturb_hf_model, prompt_ids, split_shape, weights_np
 
 pytestmark = pytest.mark.gpu
 
 
 def _cuda():
     if not torch.cuda.is_available():
-        pytest.skip("needs a B200")
+        pytest.fail("no CUDA device: the -m gpu tests must run on a B200 (there is no CPU fallback)")
 
 
 _CACHE = {}
@@ -33,8 +33,11 @@ def _setup(shape_name, B, max_length, timestamps, rows):
         return _CACHE[key]
     from oracle import hf_ref, logmel_np, whisper_np
     from taiwan_whisper_b200.synth import dequantise, synth_batch
+    shape_name, perturb = split_shape(shape_name)
     sh = SHAPES[shape_name]
     hf = hf_ref.build_hf_model(sh, seed=1234)
+    if perturb:
+        perturb_hf_model(hf)
     W = weights_np(hf)
     pcm = synth_batch(0, B)
     mel_rows = logmel_np.log_mel(dequantise(pcm[list(rows)]), sh.n_mel)
@@ -58,11 +61,11 @@ def _b200(hf, dtype, B):
 CASES = [("lv3w", 64, 256, False, (0, 1, 37, 63)), ("medw", 32, 448, True, (0, 17, 31))]
 
 
-@pytest.mark.parametrize("shape_name,B,max_length,timestamps,rows", CASES)
+@pytest.mark.parametrize("shape_name,B,max_length,timestamps,rows", CASES + [("lv3w" + PERTURBED, 64, 256, False, (0, 1, 37, 63))])
 def test_benched_width_fp32_bit_identical(shape_name, B, max_length, timestamps, rows):
     _cuda()
     from taiwan_whisper_b200.host import log_mel
-    sh = SHAPES[shape_name]
+    sh = SHAPES[split_shape(shape_name)[0]]
     hf, pcm, mel_rows, P, rules, ora = _setup(shape_name, B, max_length, timestamps, rows)
     m = _b200(hf, torch.float32, B)
     try:

@@ -9,7 +9,7 @@ import pytest
 from oracle import hf_ref, logmel_np, whisper_np
 from taiwan_whisper_b200.configs import SHAPES, token_ids
 from taiwan_whisper_b200.synth import dequantise, edge_case_clips, synth_batch
-from tests.helpers import default_rules, prompt_ids, weights_np
+from tests.helpers import default_rules, perturb_hf_model, prompt_ids, weights_np
 
 LOGMEL_TOL = 1e-4          # north_star: log-mel within 1e-4 abs
 
@@ -149,3 +149,50 @@ def test_teacher_logits_oracle_vs_golden(golden_dir, shape_name):
         top2 = np.sort(lg, axis=-1)[:, -2:]
         solid = (top2[:, 1] - top2[:, 0]) > 1e-3
         assert np.array_equal(lg.argmax(-1)[solid], g["argmax"][b][solid])
+
+
+@pytest.mark.parametrize("shape_name", ["micro80", "micro128"])
+def test_oracle_vs_hf_live_perturbed(shape_name):
+    """The oracle against a live HF fp32 forward of a model with non-trivial biases and LayerNorms (perturb_hf_model): encoder
+    output, cross-attention K / V of every decoder layer, teacher-forced logits at every position and the first greedy steps.
+    HF's init leaves biases at 0 and LayerNorms at (1, 0); the GPU tests that compare with the oracle on perturbed models rely on
+    this check."""
+    import torch
+    sh = SHAPES[shape_name]
+    hf = perturb_hf_model(hf_ref.build_hf_model(sh, seed=1234))
+    W = weights_np(hf)
+    assert np.abs(W["model.encoder.layers.1.fc1.bias"]).max() > 0.1
+    assert np.abs(W["model.decoder.layer_norm.weight"] - 1).max() > 0.1
+    mel = logmel_np.log_mel(dequantise(synth_batch(0, 2)), sh.n_mel)
+    P = prompt_ids(sh.vocab)
+    rules = default_rules(sh.vocab)
+    n_steps = 6
+
+    def rel(a, b):
+        return float(np.abs(np.asarray(a, np.float64) - b).max() / np.abs(b).max())
+
+    greedy = []
+    with torch.no_grad():
+        hf_enc = hf.model.encoder(torch.from_numpy(mel)).last_hidden_state.numpy()
+        for b in range(2):
+            enc = whisper_np.encoder_forward(W, mel[b], sh.heads, sh.enc_layers)
+            assert rel(enc, hf_enc[b]) < 1e-4, b
+            e = torch.from_numpy(hf_enc[b:b + 1])
+            for l, (k, v) in enumerate(whisper_np.cross_kv(W, hf_enc[b], sh.dec_layers)):
+                att = hf.model.decoder.layers[l].encoder_attn
+                assert rel(k, att.k_proj(e)[0].numpy()) < 1e-4, (b, l)
+                assert rel(v, att.v_proj(e)[0].numpy()) < 1e-4, (b, l)
+            toks = whisper_np.greedy_decode(W, enc, P, rules, len(P) + n_steps, sh.heads, sh.dec_layers)
+            assert len(toks) == n_steps
+            greedy.append(toks)
+            ids = P + toks
+            ref = hf(encoder_outputs=(torch.from_numpy(hf_enc[b:b + 1]),),
+                     decoder_input_ids=torch.tensor([ids])).logits[0].numpy()
+            lg = whisper_np.teacher_logits(W, enc, ids, sh.heads, sh.dec_layers)
+            assert rel(lg, ref) < 1e-4, b
+            # greedy steps: HF's argmax after the rules at every generated position is the oracle's token
+            for s in range(n_steps):
+                assert int(np.argmax(whisper_np.apply_rules(ref[len(P) - 1 + s], toks[:s], rules))) == toks[s], (b, s)
+        hf_ids = hf_ref.hf_generate(hf, mel, len(P) + n_steps)
+    for b in range(2):
+        assert hf_ids[b, :n_steps].tolist() == greedy[b], (b, hf_ids[b].tolist(), greedy[b])
