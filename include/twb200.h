@@ -307,6 +307,24 @@ TW_API int tw_debug_layernorm(tw_ctx* ctx, const float* x, const float* gamma, c
 TW_API int tw_debug_cross_kv(tw_model* m, const void* enc_out, int B, int clip0, void* stream);
 TW_API int tw_debug_read_stage1(tw_model* m, int slot, int clip0, int B, void* enc_out, int layer, void* kv_out, void* stream);
 
+/* Test entry points for the decoder as a whole, layer by layer.
+ * tw_debug_decode_taps: tw_decode_greedy (same arguments, same choice of the cross-attention path; always the launch-by-launch path,
+ *   never the CUDA graph) with
+ *   layer_tap   device float32 [n_pos, dec_layers + 1, B, d_model] or NULL: the fp32 residual after the token + position embedding
+ *               (index 0) and after every decoder layer, for decode positions pos0 .. pos0 + n_pos - 1 (prompt positions included;
+ *               need 0 <= pos0, pos0 + n_pos <= max_length - 1);
+ *   self_kv_out device [dec_layers, B, max_length - 1, 2 d_model] (model dtype) or NULL: every layer's self-attention K|V rows after
+ *               the call, read through the call's page table (rows of positions a row never reached are unspecified);
+ *   n_sms       > 0: every launch sized for a partition of that many SMs (the pipeline's decode stage); the previous count is
+ *               restored afterwards.
+ * tw_debug_decoder_logits_taps: tw_decoder_logits plus tap, device float32 [dec_layers + 1, B*T, d_model]: the fp32 residual after
+ *   the embedding and after every decoder layer. */
+TW_API int tw_debug_decode_taps(tw_model* m, const void* enc_out, int B, const int32_t* prompt, int P, const tw_rules* rules, int max_length,
+                                int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps,
+                                float* layer_tap, int pos0, int n_pos, void* self_kv_out, int n_sms, void* stream);
+TW_API int tw_debug_decoder_logits_taps(tw_model* m, const void* enc_out, int B, const int32_t* decoder_input_ids, int T, float* logits,
+                                        int64_t ld_logits, float* tap, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

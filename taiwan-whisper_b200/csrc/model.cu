@@ -524,8 +524,10 @@ int cross_kv_impl(tw_model* m, const void* enc_out, int B, cudaStream_t st, int 
 // LayerNorm kernels of the encoder at these row counts and the encoder's workspace (both passes are never in flight
 // together); attention is the encoder's tcgen05 flash kernel on separate query / key-value matrices (causal over the Tn
 // tokens, then over the K|V store), the general CUDA-core kernel in fp32 check mode.
+// tap (nullable): fp32 [L_dec + 1, B*Tn, d], the residual after the embedding and after every decoder layer.
 template <typename T>
-int decoder_logits_impl(tw_model* m, int B, const int32_t* ids, int Tn, float* logits, int64_t ld_logits, cudaStream_t st) {
+int decoder_logits_impl(tw_model* m, int B, const int32_t* ids, int Tn, float* logits, int64_t ld_logits, cudaStream_t st,
+                        float* tap = nullptr) {
     const tw_model_desc& D = m->desc;
     tw_ctx* ctx = m->ctx;
     const int d = D.d_model, V = D.vocab, M = B * Tn;
@@ -533,6 +535,7 @@ int decoder_logits_impl(tw_model* m, int B, const int32_t* ids, int Tn, float* l
     T* xn = (T*)m->ws_xn; T* qkv = (T*)m->ws_a2qkv; T* att = (T*)m->ws_att; T* hmid = (T*)m->ws_hmid; T* q = (T*)m->ws_h0;
     const size_t cross_layer = (size_t)D.max_batch * TW_N_CTX * 2 * d;
     embed_tokens_seq<T>(ids, (const T*)m->embed, (const T*)m->dec_pos, x, B, Tn, d, V, st);
+    if (tap) { copy_f32(x, tap, (int64_t)M * d, st); ctx->launches += 1; }
     for (int l = 0; l < D.dec_layers; ++l) {
         const LayerW& L = m->dec[l];
         const T* xkv = (const T*)m->xkv + l * cross_layer;
@@ -548,6 +551,7 @@ int decoder_logits_impl(tw_model* m, int B, const int32_t* ids, int Tn, float* l
         TW_CHECK(gemm<T>(m, xn, d, (const T*)L.fc1_w, d, M, D.ffn, d, mk_epi(EPI_GELU, L.fc1_b, hmid, D.ffn), st));
         TW_CHECK(gemm<T>(m, hmid, D.ffn, (const T*)L.fc2_w, D.ffn, M, d, D.ffn, mk_epi(EPI_RESID, L.fc2_b, x, d), st));
         ctx->launches += 5;       // 3 LN, 2 attention; the GEMMs count themselves
+        if (tap) { copy_f32(x, tap + (size_t)(l + 1) * M * d, (int64_t)M * d, st); ctx->launches += 1; }
     }
     layernorm<T>(x, m->dec_lnf_g, m->dec_lnf_b, xn, M, d, st);
     TW_CHECK(gemm<T>(m, xn, d, (const T*)m->embed, d, M, V, d, mk_epi(EPI_F32, nullptr, logits, ld_logits), st));
@@ -597,6 +601,7 @@ struct StepIo {
     int32_t* out_lengths;
     const int32_t* forced;
     float* logits_tap;
+    float* layer_tap;    // nullable: fp32 [L_dec + 1, B, d], the residual after the embedding and after every layer of this step
 };
 
 // Absorbed cross-attention of one decoder layer (absorb.cu): q [B, d] -> att [B, d] (the input of the output projection).
@@ -659,6 +664,8 @@ int launch_step(tw_model* m, int B, const RulesDev& R, const DecodeState& S, con
     embed_tokens<T>(S.cur_tok, (const T*)m->embed, (const T*)m->dec_pos, m->d_step, x, B, d, st);
     g_pdl = pdl_on;
     mark(-1, "embed");
+    // taps: plain stream-ordered copies (no programmatic early start), so each reads x after the kernel before it is done
+    if (io.layer_tap) { copy_f32(x, io.layer_tap, (int64_t)B * d, st); ctx->launches += 1; }
     const int32_t* pt = m->d_page_table;
     const int skip = m->skip_mask;
     for (int l = 0; l < D.dec_layers; ++l) {
@@ -668,7 +675,7 @@ int launch_step(tw_model* m, int B, const RulesDev& R, const DecodeState& S, con
         mark(l, "ln1");
         GemmEpi qe = mk_epi(EPI_STORE, L.self.qkv_b, qkv, 3 * d);
         // the K|V columns of the fused QKV projection land in the cache row of this position — only the skinny tcgen05
-        // kernel (M <= 64) implements the column split; larger batches append with a separate kernel
+        // kernel (M <= 256) implements the column split; larger batches append with a separate kernel
         const bool fused_append = (sizeof(T) == 2) && m->use_tc && m->use_tc_skinny && gemm_tc_skinny_supported(B, 3 * d, d, qe);
         if (fused_append) {
             qe.n_split = d;
@@ -714,6 +721,7 @@ int launch_step(tw_model* m, int B, const RulesDev& R, const DecodeState& S, con
         if (!(skip & 256)) TW_CHECK(gemm<T>(m, hmid, D.ffn, (const T*)L.fc2_w, D.ffn, B, d, D.ffn, mk_epi(EPI_RESID, L.fc2_b, x, d), st));
         mark(l, "fc2");
         ctx->launches += 6;       // 3 LN, self-attention, cross-attention stream + combine; the GEMMs count themselves
+        if (io.layer_tap) { copy_f32(x, io.layer_tap + (size_t)(l + 1) * B * d, (int64_t)B * d, st); ctx->launches += 1; }
     }
     layernorm<T>(x, m->dec_lnf_g, m->dec_lnf_b, xn, B, d, st);
     TW_CHECK(gemm<T>(m, xn, d, (const T*)m->embed, d, B, V, d, mk_epi(EPI_F32, nullptr, m->dlogits, m->ld_logits), st));
@@ -757,9 +765,16 @@ int begin_decode(tw_model* m, int B, const int32_t* prompt, int P, int max_lengt
     return TW_OK;
 }
 
+// Residual taps of a decode call (tw_debug_decode_taps): positions pos0 .. pos0 + n_pos - 1 into layer [n_pos, L_dec + 1, B, d].
+struct DecodeTaps {
+    float* layer = nullptr;
+    int pos0 = 0, n_pos = 0;
+};
+
 template <typename T>
 int decode_impl(tw_model* m, int B, const int32_t* prompt, int P, const RulesDev& R, int max_length, int32_t* out_tokens,
-                int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps, cudaStream_t st) {
+                int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps, cudaStream_t st,
+                const DecodeTaps& taps = DecodeTaps{}) {
     tw_ctx* ctx = m->ctx;
     const int n_gen_max = max_length - P;
     DecodeState S;
@@ -776,10 +791,10 @@ int decode_impl(tw_model* m, int B, const int32_t* prompt, int P, const RulesDev
     }
 
     // CUDA graph of one step: production path only (no teacher forcing / taps / per-launch profiling events)
-    const bool want_graph = m->use_graph && !forced && !logits_tap && !m->prof_on && m->trace_pos < 0;
+    const bool want_graph = m->use_graph && !forced && !logits_tap && !taps.layer && !m->prof_on && m->trace_pos < 0;
     // the graph bakes in its output pointers: decode into the model-owned buffers, copy out at the end
-    StepIo io{out_tokens, out_lengths, forced, logits_tap};
-    if (want_graph) io = StepIo{m->d_out_tok, m->d_out_len, nullptr, nullptr};
+    StepIo io{out_tokens, out_lengths, forced, logits_tap, nullptr};
+    if (want_graph) io = StepIo{m->d_out_tok, m->d_out_len, nullptr, nullptr, nullptr};
     if (want_graph) TW_CUDA_OK(ctx, cudaMemsetAsync(m->d_out_len, 0, B * sizeof(int32_t), st));
     m->skip_mask = getenv("TWB200_SKIP") ? atoi(getenv("TWB200_SKIP")) : 0;      // re-read per call: one process can sweep masks
     GraphKey key{B, R.eos, R.pad, R.ts_begin, R.no_timestamps, R.max_initial_ts, (m->row_budget_on ? 1 : 0) | (m->skip_mask << 1),
@@ -826,6 +841,8 @@ int decode_impl(tw_model* m, int B, const int32_t* prompt, int P, const RulesDev
             TW_CUDA_OK(ctx, cudaGraphLaunch(exec, st));
             ctx->launches += exec_kernels;
         } else {
+            const bool tapped = taps.layer && pos >= taps.pos0 && pos < taps.pos0 + taps.n_pos;
+            io.layer_tap = tapped ? taps.layer + (size_t)(pos - taps.pos0) * (m->desc.dec_layers + 1) * B * m->desc.d_model : nullptr;
             TW_CHECK(launch_step<T>(m, B, R, S, io, st, pos == m->trace_pos));
         }
         ++steps_done;
@@ -1092,6 +1109,25 @@ static int check_decode_args(tw_model* m, int B, const int32_t* prompt, int P, c
     return TW_OK;
 }
 
+// tw_decode_greedy after its argument checks; tw_debug_decode_taps adds residual taps
+static int decode_greedy_call(tw_model* m, const void* enc_out, int B, const int32_t* prompt, int P, const tw_rules* rules, int max_length,
+                              int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps,
+                              cudaStream_t st, const DecodeTaps& taps) {
+    RulesDev R;
+    TW_CHECK(upload_rules(m, rules, &R, st));
+    cudaEventRecord(m->ev[2], st);
+    int r = cross_kv_for_decode(m, enc_out, B, st);
+    if (r != TW_OK) return r;
+    cudaEventRecord(m->ev[3], st);
+    r = m->desc.dtype == TW_BF16
+            ? decode_impl<__nv_bfloat16>(m, B, prompt, P, R, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps, st, taps)
+            : decode_impl<float>(m, B, prompt, P, R, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps, st, taps);
+    cudaEventRecord(m->ev[4], st);
+    m->ev_valid[2] = m->ev_valid[3] = m->ev_valid[4] = true;
+    m->ev_valid[0] = m->ev_valid[1] = m->ev_valid[6] = m->ev_valid[7] = false;
+    return r;
+}
+
 int tw_decode_greedy(tw_model* m, const void* enc_out, int B, const int32_t* prompt, int P, const tw_rules* rules, int max_length,
                      int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps,
                      void* stream) {
@@ -1101,24 +1137,52 @@ int tw_decode_greedy(tw_model* m, const void* enc_out, int B, const int32_t* pro
         m->ctx->set_error(TW_E_INVALID, "tw_decode_greedy: null buffer");
         return TW_E_INVALID;
     }
-    cudaStream_t st = (cudaStream_t)stream;
-    RulesDev R;
-    TW_CHECK(upload_rules(m, rules, &R, st));
-    cudaEventRecord(m->ev[2], st);
-    int r = cross_kv_for_decode(m, enc_out, B, st);
-    if (r != TW_OK) return r;
-    cudaEventRecord(m->ev[3], st);
-    r = m->desc.dtype == TW_BF16
-            ? decode_impl<__nv_bfloat16>(m, B, prompt, P, R, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps, st)
-            : decode_impl<float>(m, B, prompt, P, R, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps, st);
-    cudaEventRecord(m->ev[4], st);
-    m->ev_valid[2] = m->ev_valid[3] = m->ev_valid[4] = true;
-    m->ev_valid[0] = m->ev_valid[1] = m->ev_valid[6] = m->ev_valid[7] = false;
-    return r;
+    return decode_greedy_call(m, enc_out, B, prompt, P, rules, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps,
+                              (cudaStream_t)stream, DecodeTaps{});
 }
 
-int tw_decoder_logits(tw_model* m, const void* enc_out, int B, const int32_t* decoder_input_ids, int T, float* logits,
-                      int64_t ld_logits, void* stream) {
+int tw_debug_decode_taps(tw_model* m, const void* enc_out, int B, const int32_t* prompt, int P, const tw_rules* rules, int max_length,
+                         int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps,
+                         float* layer_tap, int pos0, int n_pos, void* self_kv_out, int n_sms, void* stream) {
+    if (!check_model(m, "tw_debug_decode_taps")) return TW_E_INVALID;
+    TW_CHECK(check_decode_args(m, B, prompt, P, rules, max_length));
+    tw_ctx* ctx = m->ctx;
+    if (!enc_out || !out_tokens || !out_lengths || (layer_tap && (pos0 < 0 || n_pos < 0 || pos0 + n_pos > max_length - 1)) || n_sms < 0) {
+        ctx->set_error(TW_E_INVALID, "tw_debug_decode_taps: null buffer, tapped positions outside 0 .. max_length - 2 or n_sms < 0");
+        return TW_E_INVALID;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    DecodeTaps taps;
+    taps.layer = layer_tap;
+    taps.pos0 = pos0;
+    taps.n_pos = layer_tap ? n_pos : 0;
+    // every launch sized for a partition of n_sms SMs, as the pipeline's decode stage sizes them
+    const int sms_before = ctx->sm_count;
+    const int da_before = decode_attention_set_sms(n_sms);
+    if (n_sms > 0) ctx->sm_count = n_sms;
+    int r = decode_greedy_call(m, enc_out, B, prompt, P, rules, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps, st, taps);
+    decode_attention_set_sms(da_before);
+    ctx->sm_count = sms_before;
+    if (r != TW_OK || !self_kv_out) return r;
+    // the self-attention K|V rows of positions 0 .. max_length - 2, read through the page table this call wrote
+    const tw_model_desc& D = m->desc;
+    const size_t e = m->esz, row = 2 * (size_t)D.d_model * e, n_rows = max_length - 1;
+    const size_t self_layer = (size_t)D.max_batch * m->kv_pages * TW_KV_PAGE * row;
+    for (int l = 0; l < D.dec_layers; ++l)
+        for (int b = 0; b < B; ++b)
+            for (size_t p0 = 0; p0 < n_rows; p0 += TW_KV_PAGE) {
+                const int page = m->h_page_table[b * m->kv_pages + p0 / TW_KV_PAGE];
+                const size_t rows = n_rows - p0 < (size_t)TW_KV_PAGE ? n_rows - p0 : (size_t)TW_KV_PAGE;
+                const char* src = (const char*)m->self_kv + l * self_layer + (size_t)page * TW_KV_PAGE * row;
+                char* dst = (char*)self_kv_out + (((size_t)l * B + b) * n_rows + p0) * row;
+                TW_CUDA_OK(ctx, cudaMemcpyAsync(dst, src, rows * row, cudaMemcpyDeviceToDevice, st));
+            }
+    return TW_OK;
+}
+
+// tw_decoder_logits with an optional residual tap (tw_debug_decoder_logits_taps)
+static int decoder_logits_call(tw_model* m, const void* enc_out, int B, const int32_t* decoder_input_ids, int T, float* logits,
+                               int64_t ld_logits, cudaStream_t st, float* tap) {
     if (!check_model(m, "tw_decoder_logits")) return TW_E_INVALID;
     tw_ctx* ctx = m->ctx;
     if (B <= 0 || B > m->desc.max_batch || !enc_out || !decoder_input_ids || !logits) {
@@ -1134,11 +1198,24 @@ int tw_decoder_logits(tw_model* m, const void* enc_out, int B, const int32_t* de
         ctx->set_error(TW_E_INVALID, "tw_decoder_logits: logits need a 16-byte aligned base and a row pitch >= vocab that is a multiple of 4 floats");
         return TW_E_INVALID;
     }
-    cudaStream_t st = (cudaStream_t)stream;
     int r = m->desc.dtype == TW_BF16 ? cross_kv_impl<__nv_bfloat16>(m, enc_out, B, st) : cross_kv_impl<float>(m, enc_out, B, st);
     if (r != TW_OK) return r;
-    return m->desc.dtype == TW_BF16 ? decoder_logits_impl<__nv_bfloat16>(m, B, decoder_input_ids, T, logits, ld_logits, st)
-                                    : decoder_logits_impl<float>(m, B, decoder_input_ids, T, logits, ld_logits, st);
+    return m->desc.dtype == TW_BF16 ? decoder_logits_impl<__nv_bfloat16>(m, B, decoder_input_ids, T, logits, ld_logits, st, tap)
+                                    : decoder_logits_impl<float>(m, B, decoder_input_ids, T, logits, ld_logits, st, tap);
+}
+
+int tw_decoder_logits(tw_model* m, const void* enc_out, int B, const int32_t* decoder_input_ids, int T, float* logits,
+                      int64_t ld_logits, void* stream) {
+    return decoder_logits_call(m, enc_out, B, decoder_input_ids, T, logits, ld_logits, (cudaStream_t)stream, nullptr);
+}
+
+int tw_debug_decoder_logits_taps(tw_model* m, const void* enc_out, int B, const int32_t* decoder_input_ids, int T, float* logits,
+                                 int64_t ld_logits, float* tap, void* stream) {
+    if (m && !tap) {
+        m->ctx->set_error(TW_E_INVALID, "tw_debug_decoder_logits_taps: null tap");
+        return TW_E_INVALID;
+    }
+    return decoder_logits_call(m, enc_out, B, decoder_input_ids, T, logits, ld_logits, (cudaStream_t)stream, tap);
 }
 
 int tw_transcribe_host(tw_model* m, const int16_t* pcm_host, const int32_t* n_valid_host, int B, const int32_t* prompt, int P,

@@ -156,8 +156,8 @@ def _model(shape_name):
 
 @functools.lru_cache(maxsize=None)
 def _weights64(shape_name, rounded):
-    """float64 device copies of the encoder / cross-K|V weights: as the model holds them (rounded: bf16 matrices, q rows and q
-    bias scaled by 0.125) or exactly as HF holds them (the unrounded fp64 run)."""
+    """float64 device copies of the encoder / decoder weights: as the model holds them (rounded: bf16 matrices, token embedding and
+    decoder positions, q rows and q bias scaled by 0.125) or exactly as HF holds them (the unrounded fp64 run)."""
     from tests.gpu_common import hf_model
     sd = {k: v.detach().to("cuda", torch.float64) for k, v in hf_model(shape_name, 1234, True).state_dict().items()}
     sh = SHAPES[shape_name]
@@ -180,6 +180,24 @@ def _weights64(shape_name, rounded):
         a = f"model.decoder.layers.{l}.encoder_attn."
         W["kv"].append(dict(w=torch.cat([r(sd[a + "k_proj.weight"]), r(sd[a + "v_proj.weight"])]),
                             b=torch.cat([torch.zeros_like(sd[a + "v_proj.bias"]), sd[a + "v_proj.bias"]])))
+    # decoder: the self-attention and MLP as in the encoder, the cross-attention q projection and out projection (its K|V
+    # projection is W["kv"]), layer norms 1 / 2 / 3 in front of self-attention / cross-attention / MLP
+    Dc = "model.decoder."
+    W.update(embed=r(sd[Dc + "embed_tokens.weight"]), dec_pos=r(sd[Dc + "embed_positions.weight"]),
+             dlnf_g=sd[Dc + "layer_norm.weight"], dlnf_b=sd[Dc + "layer_norm.bias"], dec=[])
+    for l in range(sh.dec_layers):
+        p = f"{Dc}layers.{l}."
+        a, c = p + "self_attn.", p + "encoder_attn."
+        W["dec"].append(dict(
+            ln1_g=sd[p + "self_attn_layer_norm.weight"], ln1_b=sd[p + "self_attn_layer_norm.bias"],
+            wqkv=torch.cat([r(0.125 * sd[a + "q_proj.weight"]), r(sd[a + "k_proj.weight"]), r(sd[a + "v_proj.weight"])]),
+            bqkv=torch.cat([0.125 * sd[a + "q_proj.bias"], torch.zeros_like(sd[a + "v_proj.bias"]), sd[a + "v_proj.bias"]]),
+            wo=r(sd[a + "out_proj.weight"]), bo=sd[a + "out_proj.bias"],
+            ln2_g=sd[p + "encoder_attn_layer_norm.weight"], ln2_b=sd[p + "encoder_attn_layer_norm.bias"],
+            wq_c=r(0.125 * sd[c + "q_proj.weight"]), bq_c=0.125 * sd[c + "q_proj.bias"],
+            wkv_c=W["kv"][l]["w"], bkv_c=W["kv"][l]["b"], wo_c=r(sd[c + "out_proj.weight"]), bo_c=sd[c + "out_proj.bias"],
+            ln3_g=sd[p + "final_layer_norm.weight"], ln3_b=sd[p + "final_layer_norm.bias"],
+            w1=r(sd[p + "fc1.weight"]), b1=sd[p + "fc1.bias"], w2=r(sd[p + "fc2.weight"]), b2=sd[p + "fc2.bias"]))
     return W
 
 
