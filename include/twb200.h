@@ -131,7 +131,8 @@ typedef struct {
  * 30 s window per row.
  *   enc_out     device [B,1500,d] model dtype (from tw_encode)
  *   prompt      host int32 [P]: forced tokens <|sot|><|zh|><|transcribe|>[<|notimestamps|>]
- *               (_retrieve_init_tokens, generation_whisper.py:1455-1608), same for every row
+ *               (_retrieve_init_tokens, generation_whisper.py:1455-1608), same for every row (per-row prompts and language
+ *               detection: tw_decode_greedy_rows below)
  *   max_length  total length incl. prompt (HF max_length); P < max_length <= max_target
  *   out_tokens  device int32 [B, max_length - P]: generated ids; after a row's EOS: pad
  *   out_lengths device int32 [B]: number of generated tokens before EOS
@@ -142,6 +143,36 @@ TW_API int tw_decode_greedy(tw_model* m, const void* enc_out, int B, const int32
                      int max_length, int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced,
                      float* logits_tap, int tap_steps, void* stream);
 
+/* ---- per-row prompts and language detection
+ * HF builds one forced prompt per row (_retrieve_init_tokens, generation_whisper.py:1455-1608): a `language` list gives each row its
+ * own language, and language=None detects it (detect_language, :1610-1673: the logits of the step fed <|startoftranscript|>,
+ * every id outside lang_to_id at -inf, argmax).  Here the detection is taken inside step 0 of the decode itself — that step is
+ * fed SOT and produces exactly those logits — so it costs no second decoder pass.
+ *   prompts   host int32 [B][P]: row b's forced tokens; all rows start with the same token (SOT); -1 at index 1 = detect this
+ *             row's language there.  P <= 24.
+ *   lang_ids  host int32 [n_lang] (1 <= n_lang <= 128): the ids detection chooses among (the lang_to_id values: 99 or 100);
+ *             NULL when no row detects.  Ties go to the smallest id, as torch.argmax over the masked row.
+ *   out_lang  [B] or NULL: the language id each row was decoded with (its prompt token 1, detected or given).  A device buffer
+ *             for tw_decode_greedy_rows / tw_debug_select_steps_rows, a HOST buffer for tw_transcribe_host_rows /
+ *             tw_pipeline_decode_rows (filled before they return).  Needs P >= 2.
+ * The _rows variants take the arguments of their single-prompt forms with `prompt` replaced by `rows`; the single-prompt forms
+ * are the _rows forms with their prompt given to every row. */
+typedef struct {
+    const int32_t* prompts;   /* host [B][P]; -1 at index 1 = detect this row's language */
+    const int32_t* lang_ids;  /* host [n_lang]; ids detection chooses among (NULL when no row detects) */
+    int32_t n_lang;
+    int32_t* out_lang;        /* [B] device, or NULL: the language id each row was decoded with */
+} tw_prompt_rows;
+
+TW_API int tw_decode_greedy_rows(tw_model* m, const void* enc_out, int B, const tw_prompt_rows* rows, int P, const tw_rules* rules,
+                                 int max_length, int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced,
+                                 float* logits_tap, int tap_steps, void* stream);
+/* Replaces WhisperGenerationMixin.detect_language: the language id of every row of enc_out [B,1500,d] (device, model dtype; from
+ * tw_encode) into out_lang (device int32 [B]) — step 0 of a decode fed <|startoftranscript|> (50258), then the pick over lang_ids
+ * (host int32 [n_lang]). */
+TW_API int tw_detect_language(tw_model* m, const void* enc_out, int B, const int32_t* lang_ids, int n_lang, int32_t* out_lang,
+                              void* stream);
+
 /* The whole path with HOST buffers: pinned (or pageable) int16 PCM in, token ids out —
  * H2D copy, log-mel, encoder, cross-K/V, greedy decode, D2H copy, stream-synchronised on return.
  * One call = the reference's feature_extractor(...) + model.generate(...) for a batch.
@@ -150,6 +181,9 @@ TW_API int tw_decode_greedy(tw_model* m, const void* enc_out, int B, const int32
 TW_API int tw_transcribe_host(tw_model* m, const int16_t* pcm_host, const int32_t* n_valid_host, int B,
                        const int32_t* prompt, int P, const tw_rules* rules, int max_length,
                        int32_t* out_tokens_host, int32_t* out_lengths_host, void* stream);
+TW_API int tw_transcribe_host_rows(tw_model* m, const int16_t* pcm_host, const int32_t* n_valid_host, int B,
+                                   const tw_prompt_rows* rows, int P, const tw_rules* rules, int max_length,
+                                   int32_t* out_tokens_host, int32_t* out_lengths_host, void* stream);
 
 /* Two-stage pipeline over SM partitions: the batch loop of the reference (ref training/run_pseudo_labelling.py:915-918,
  * `for step, (batch, file_ids) in enumerate(...): generated_ids = generate_fn(batch["input_features"], **gen_kwargs)`) handles one
@@ -184,6 +218,8 @@ TW_API int tw_pipeline_encode(tw_model* m, const int16_t* pcm, const int32_t* n_
 TW_API int tw_pipeline_encode_at(tw_model* m, const int16_t* pcm, const int32_t* n_valid_host, int B, int slot, int clip0);
 TW_API int tw_pipeline_decode(tw_model* m, int slot, int B, const int32_t* prompt, int P, const tw_rules* rules, int max_length,
                               int32_t* out_tokens_host, int32_t* out_lengths_host);
+TW_API int tw_pipeline_decode_rows(tw_model* m, int slot, int B, const tw_prompt_rows* rows, int P, const tw_rules* rules,
+                                   int max_length, int32_t* out_tokens_host, int32_t* out_lengths_host);
 
 /* Per-stage device time of the last tw_transcribe_host / tw_decode_greedy call in ms (CUDA events on the call's
  * stream): [0] log-mel, [1] encoder, [2] cross-K/V, [3] decode (incl. the D2H of the ids), [4] total, [5] H2D copy. */
@@ -282,6 +318,12 @@ TW_API int tw_debug_encoder_attention(tw_ctx* ctx, const void* qkv, void* out, i
 TW_API int tw_debug_select_steps(tw_model* m, const float* logits, int64_t ld_logits, int B, const int32_t* prompt, int P,
                                  const tw_rules* rules, int max_length, const int32_t* row_budgets, const int32_t* forced, float* logits_tap,
                                  int tap_steps, int32_t* out_tokens, int32_t* out_lengths, int32_t* n_active, int32_t* active, void* stream);
+/* tw_debug_select_steps with per-row prompts: when a row detects (or out_lang is given), position 0 runs the language pick of
+ * tw_decode_greedy_rows on the step-0 logits (logits + 0) in place of the selection. */
+TW_API int tw_debug_select_steps_rows(tw_model* m, const float* logits, int64_t ld_logits, int B, const tw_prompt_rows* rows, int P,
+                                      const tw_rules* rules, int max_length, const int32_t* row_budgets, const int32_t* forced,
+                                      float* logits_tap, int tap_steps, int32_t* out_tokens, int32_t* out_lengths, int32_t* n_active,
+                                      int32_t* active, void* stream);
 TW_API int tw_debug_kv_append(tw_ctx* ctx, const void* A, const void* W, const float* bias, void* C, void* pool, const int32_t* page_table,
                               int pt_stride, const int32_t* d_pos, int M, int d, int dtype, int fused, int n_sms, void* stream);
 TW_API int tw_debug_self_attention_step(tw_ctx* ctx, const void* q, int64_t q_stride, const void* kv, int64_t kv_clip_stride,

@@ -82,8 +82,10 @@ void im2col_conv2(const T* h0, T* out, int B, int d, cudaStream_t st);
 struct DecodeState;
 // Decode-step state lives on the device so that one captured CUDA graph can be replayed for every token:
 //   d_step[0] = pos (position of the token being fed), [1] = P (prompt length), [2] = stride of out_tokens,
-//   [3] = number of steps whose post-rules logits are tapped, [8 .. 8+P) = forced prompt tokens.
-constexpr int STEP_POS = 0, STEP_P = 1, STEP_STRIDE = 2, STEP_TAP = 3, STEP_PROMPT = 8, STEP_INTS = 32;
+//   [3] = number of steps whose post-rules logits are tapped.  The forced prompt tokens are per row (DecodeState::prompt).
+constexpr int STEP_POS = 0, STEP_P = 1, STEP_STRIDE = 2, STEP_TAP = 3, STEP_INTS = 8;
+// row b's forced prompt occupies prompt[b * PROMPT_MAX .. b * PROMPT_MAX + P); PROMPT_DETECT at index 1 = detect the language
+constexpr int PROMPT_MAX = 24, PROMPT_DETECT = -1, MAX_LANG_IDS = 128;
 // x[b] = E[tok[b]] + P[pos]   (f32 residual stream)
 template <typename T>
 void embed_tokens(const int32_t* tok, const T* E, const T* P, const int32_t* d_step, float* x, int B, int d, cudaStream_t st);
@@ -165,11 +167,16 @@ struct DecodeState {
     // optional per-row budget of generated tokens (test / bench hook, tw_debug_set_row_budgets): row b finishes after
     // row_budget[b] tokens exactly as if it had emitted EOS there; null = off
     const int32_t* row_budget;
+    int32_t* prompt;      // [max_batch][PROMPT_MAX] forced prompt of every row (slot 1 is rewritten by the language pick)
 };
 // one CTA per row: rules -> argmax -> finished/pad bookkeeping -> next input token
 // (inside the forced prompt it only feeds the next prompt token)
 void select_tokens(const float* logits, int64_t ld_logits, int V, int B, const int32_t* d_step, const RulesDev& rules, const DecodeState& st,
                    int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced, float* logits_tap, cudaStream_t stream);
+// the language pick of step 0 (in place of select_tokens there): row b whose prompt slot 1 is PROMPT_DETECT takes the argmax of its
+// logits over lang_ids (first id wins ties); every row then feeds its slot 1, and out_lang[b] (nullable) records it
+void pick_language(const float* logits, int64_t ld_logits, int B, const int32_t* lang_ids, int n_lang, const DecodeState& st,
+                   int32_t* out_lang, cudaStream_t stream);
 void decode_state_init(const DecodeState& st, int B, int first_tok, cudaStream_t stream);
 void set_cur_tok(const DecodeState& st, int B, int tok, cudaStream_t stream);
 

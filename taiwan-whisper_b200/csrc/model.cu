@@ -145,6 +145,14 @@ struct tw_model {
     int32_t* h_flag = nullptr;   // pinned
     int32_t* h_step = nullptr;   // pinned staging of the step header
     int32_t* d_step = nullptr;   // device step state (kernels.cuh STEP_*)
+    // per-row forced prompts [max_batch][PROMPT_MAX] and the language ids detection chooses among, rewritten per decode call
+    // from pinned staging (h_rows: the prompt table, then MAX_LANG_IDS ids); d_out_lang: languages of the host-output calls
+    int32_t* d_row_prompt = nullptr;
+    int32_t* d_lang_ids = nullptr;
+    int32_t* h_rows = nullptr;
+    int32_t* d_out_lang = nullptr;
+    int n_lang_now = 0;          // language ids of the decode call in progress
+    bool pick_now = false;       // its step 0 runs the language pick in place of the selection
     bool use_graph = true;       // replay one captured CUDA graph per decode step
     bool use_pdl = true;         // programmatic dependent launch inside the decode step
     cudaStream_t cap_stream = nullptr;
@@ -403,6 +411,10 @@ int alloc_workspace(tw_model* m) {
     TW_CUDA_OK(m->ctx, cudaMallocHost(&m->h_flag, 64));
     TW_CUDA_OK(m->ctx, cudaMallocHost(&m->h_step, STEP_INTS * sizeof(int32_t)));
     TW_CHECK(dev_alloc(m, (void**)&m->d_step, STEP_INTS * sizeof(int32_t)));
+    TW_CHECK(dev_alloc(m, (void**)&m->d_row_prompt, (B * PROMPT_MAX + MAX_LANG_IDS) * sizeof(int32_t)));
+    m->d_lang_ids = m->d_row_prompt + B * PROMPT_MAX;
+    TW_CUDA_OK(m->ctx, cudaMallocHost(&m->h_rows, (B * PROMPT_MAX + MAX_LANG_IDS) * sizeof(int32_t)));
+    TW_CHECK(dev_alloc(m, (void**)&m->d_out_lang, B * sizeof(int32_t)));
     TW_CUDA_OK(m->ctx, cudaStreamCreateWithFlags(&m->cap_stream, cudaStreamNonBlocking));
     return TW_OK;
 }
@@ -602,6 +614,7 @@ struct StepIo {
     const int32_t* forced;
     float* logits_tap;
     float* layer_tap;    // nullable: fp32 [L_dec + 1, B, d], the residual after the embedding and after every layer of this step
+    int32_t* out_lang;   // nullable: [B] the language each row is decoded with (written by the language pick of step 0)
 };
 
 // Absorbed cross-attention of one decoder layer (absorb.cu): q [B, d] -> att [B, d] (the input of the output projection).
@@ -635,7 +648,10 @@ int cross_absorbed<__nv_bfloat16>(tw_model* m, const LayerW& L, const __nv_bfloa
 // One decode step (all kernels of one token position).  Position, prompt and output stride are read from
 // m->d_step on the device, so the same launch sequence — or one captured CUDA graph — serves every position.
 template <typename T>
-int launch_step(tw_model* m, int B, const RulesDev& R, const DecodeState& S, const StepIo& io, cudaStream_t st, bool trace = false) {
+// pick: step 0 of a call that detects languages (or reports them) — the language pick replaces the token selection.  Step 0 is
+// always launched eagerly (the graph is captured at pos >= 1), so the replayed step never contains the pick.
+int launch_step(tw_model* m, int B, const RulesDev& R, const DecodeState& S, const StepIo& io, cudaStream_t st, bool pick = false,
+                bool trace = false) {
     const tw_model_desc& D = m->desc;
     tw_ctx* ctx = m->ctx;
     const int d = D.d_model, V = D.vocab, H = D.heads;
@@ -725,22 +741,20 @@ int launch_step(tw_model* m, int B, const RulesDev& R, const DecodeState& S, con
     }
     layernorm<T>(x, m->dec_lnf_g, m->dec_lnf_b, xn, B, d, st);
     TW_CHECK(gemm<T>(m, xn, d, (const T*)m->embed, d, B, V, d, mk_epi(EPI_F32, nullptr, m->dlogits, m->ld_logits), st));
-    select_tokens(m->dlogits, m->ld_logits, V, B, m->d_step, R, S, io.out_tokens, io.out_lengths, io.forced, io.logits_tap, st);
+    if (pick) pick_language(m->dlogits, m->ld_logits, B, m->d_lang_ids, m->n_lang_now, S, io.out_lang, st);
+    else select_tokens(m->dlogits, m->ld_logits, V, B, m->d_step, R, S, io.out_tokens, io.out_lengths, io.forced, io.logits_tap, st);
     advance_step(m->d_step, S, B, st);
-    ctx->launches += 4;           // embed, LN, select, advance
+    ctx->launches += 4;           // embed, LN, select (or the language pick), advance
     return TW_OK;
 }
 
-// Decode state of one call (the model's dstate arrays, initialised for B rows), the cleared out_lengths and the step header
-// (position 0, prompt, output stride, tapped steps) on the device: shared by decode_impl and tw_debug_select_steps.
-int begin_decode(tw_model* m, int B, const int32_t* prompt, int P, int max_length, int32_t* out_lengths, float* logits_tap, int tap_steps,
-                 cudaStream_t st, DecodeState* out) {
+// Decode state of one call (the model's dstate arrays, initialised for B rows), the cleared out_lengths, the step header (position 0,
+// prompt length, output stride, tapped steps), the per-row prompt table and the language ids on the device: shared by decode_impl and
+// tw_debug_select_steps.  rows.prompts is host [B][P] (checked by check_prompt_rows).
+int begin_decode(tw_model* m, int B, const tw_prompt_rows& rows, int P, int max_length, int32_t* out_lengths, float* logits_tap,
+                 int tap_steps, cudaStream_t st, DecodeState* out) {
     const tw_model_desc& D = m->desc;
     tw_ctx* ctx = m->ctx;
-    if (P > STEP_INTS - STEP_PROMPT) {
-        ctx->set_error(TW_E_INVALID, "decode: prompt longer than 24 tokens is not supported");
-        return TW_E_INVALID;
-    }
     DecodeState& S = *out;
     S.cur_tok = m->dstate;
     S.finished = m->dstate + D.max_batch;
@@ -752,15 +766,31 @@ int begin_decode(tw_model* m, int B, const int32_t* prompt, int P, int max_lengt
     S.row_budget = m->row_budget_on ? m->d_row_budget : nullptr;
     S.n_unfinished = m->dstate + 8 * D.max_batch;
     S.n_active = m->dstate + 8 * D.max_batch + 1;
-    decode_state_init(S, B, prompt[0], st);
+    S.prompt = m->d_row_prompt;
+    decode_state_init(S, B, rows.prompts[0], st);          // SOT: the same in every row
     TW_CUDA_OK(ctx, cudaMemsetAsync(out_lengths, 0, B * sizeof(int32_t), st));
     // step header -> device (pinned staging so the copy is stream-ordered)
     int32_t* hs = m->h_step;
     TW_CUDA_OK(ctx, cudaStreamSynchronize(st));          // previous call may still be reading h_step
     for (int i = 0; i < STEP_INTS; ++i) hs[i] = 0;
     hs[STEP_POS] = 0; hs[STEP_P] = P; hs[STEP_STRIDE] = max_length - P; hs[STEP_TAP] = logits_tap ? tap_steps : 0;
-    for (int i = 0; i < P; ++i) hs[STEP_PROMPT + i] = prompt[i];
     TW_CUDA_OK(ctx, cudaMemcpyAsync(m->d_step, hs, STEP_INTS * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    // prompt table (rows B .. max_batch - 1 are not read) and language ids, from pinned staging like the step header
+    int32_t* hp = m->h_rows;
+    bool detect = false;
+    for (int b = 0; b < B; ++b)
+        for (int i = 0; i < PROMPT_MAX; ++i) {
+            hp[b * PROMPT_MAX + i] = i < P ? rows.prompts[(size_t)b * P + i] : 0;
+            detect |= (i == 1 && i < P && hp[b * PROMPT_MAX + i] == PROMPT_DETECT);
+        }
+    TW_CUDA_OK(ctx, cudaMemcpyAsync(m->d_row_prompt, hp, (size_t)B * PROMPT_MAX * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    m->n_lang_now = rows.lang_ids ? rows.n_lang : 0;
+    if (m->n_lang_now > 0) {
+        int32_t* hl = hp + D.max_batch * PROMPT_MAX;
+        for (int j = 0; j < m->n_lang_now; ++j) hl[j] = rows.lang_ids[j];
+        TW_CUDA_OK(ctx, cudaMemcpyAsync(m->d_lang_ids, hl, m->n_lang_now * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+    }
+    m->pick_now = detect || rows.out_lang;
     ctx->launches += 1;
     return TW_OK;
 }
@@ -772,13 +802,13 @@ struct DecodeTaps {
 };
 
 template <typename T>
-int decode_impl(tw_model* m, int B, const int32_t* prompt, int P, const RulesDev& R, int max_length, int32_t* out_tokens,
+int decode_impl(tw_model* m, int B, const tw_prompt_rows& rows, int P, const RulesDev& R, int max_length, int32_t* out_tokens,
                 int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps, cudaStream_t st,
                 const DecodeTaps& taps = DecodeTaps{}) {
     tw_ctx* ctx = m->ctx;
     const int n_gen_max = max_length - P;
     DecodeState S;
-    TW_CHECK(begin_decode(m, B, prompt, P, max_length, out_lengths, logits_tap, tap_steps, st, &S));
+    TW_CHECK(begin_decode(m, B, rows, P, max_length, out_lengths, logits_tap, tap_steps, st, &S));
     // page table of this call: only the ceil(max_length / TW_KV_PAGE) pages a clip can reach are mapped, page-major
     // (logical page p of clip b -> physical page p*B + b), so a call touches a dense prefix of every layer's pool whose
     // size follows B and max_length, and the B cache rows written by one step are adjacent
@@ -793,8 +823,8 @@ int decode_impl(tw_model* m, int B, const int32_t* prompt, int P, const RulesDev
     // CUDA graph of one step: production path only (no teacher forcing / taps / per-launch profiling events)
     const bool want_graph = m->use_graph && !forced && !logits_tap && !taps.layer && !m->prof_on && m->trace_pos < 0;
     // the graph bakes in its output pointers: decode into the model-owned buffers, copy out at the end
-    StepIo io{out_tokens, out_lengths, forced, logits_tap, nullptr};
-    if (want_graph) io = StepIo{m->d_out_tok, m->d_out_len, nullptr, nullptr, nullptr};
+    StepIo io{out_tokens, out_lengths, forced, logits_tap, nullptr, rows.out_lang};
+    if (want_graph) io = StepIo{m->d_out_tok, m->d_out_len, nullptr, nullptr, nullptr, rows.out_lang};
     if (want_graph) TW_CUDA_OK(ctx, cudaMemsetAsync(m->d_out_len, 0, B * sizeof(int32_t), st));
     m->skip_mask = getenv("TWB200_SKIP") ? atoi(getenv("TWB200_SKIP")) : 0;      // re-read per call: one process can sweep masks
     GraphKey key{B, R.eos, R.pad, R.ts_begin, R.no_timestamps, R.max_initial_ts, (m->row_budget_on ? 1 : 0) | (m->skip_mask << 1),
@@ -843,7 +873,7 @@ int decode_impl(tw_model* m, int B, const int32_t* prompt, int P, const RulesDev
         } else {
             const bool tapped = taps.layer && pos >= taps.pos0 && pos < taps.pos0 + taps.n_pos;
             io.layer_tap = tapped ? taps.layer + (size_t)(pos - taps.pos0) * (m->desc.dec_layers + 1) * B * m->desc.d_model : nullptr;
-            TW_CHECK(launch_step<T>(m, B, R, S, io, st, pos == m->trace_pos));
+            TW_CHECK(launch_step<T>(m, B, R, S, io, st, pos == 0 && m->pick_now, pos == m->trace_pos));
         }
         ++steps_done;
         const int g = pos - (P - 1);
@@ -887,6 +917,9 @@ int decode_impl(tw_model* m, int B, const int32_t* prompt, int P, const RulesDev
     TW_CUDA_OK(ctx, cudaGetLastError());
     return TW_OK;
 }
+
+// <|startoftranscript|> of the multilingual Whisper vocabularies (51865 and 51866 ids), the token detection feeds
+constexpr int WHISPER_SOT = 50258;
 
 bool check_model(tw_model* m, const char* fn) {
     return m && m->ctx && fn;
@@ -1069,7 +1102,8 @@ size_t tw_workspace_bytes(const tw_model_desc* desc) {
                 al((size_t)D.dec_layers * B * kv_pages * TW_KV_PAGE * 2 * d * e) + al(B * kv_pages * sizeof(int32_t)) +
                 al(B * d * f4) + al(B * d * e) + al(B * 3 * d * e) + al(B * d * e) + al(B * d * e) + al(B * ffn * e) + al(B * ((V + 3) / 4 * 4) * f4) +
                 al(decode_attention_partial_floats((int)B, D.heads) * f4) + al((8 * B + 8) * sizeof(int32_t)) + al(V + 16) + al(V + 16) +
-                al(4096 * sizeof(int32_t)) + al(B * D.max_target * sizeof(int32_t)) + al(B * sizeof(int32_t)) + al(STEP_INTS * sizeof(int32_t));
+                al(4096 * sizeof(int32_t)) + al(B * D.max_target * sizeof(int32_t)) + al(B * sizeof(int32_t)) + al(STEP_INTS * sizeof(int32_t)) +
+                al((B * PROMPT_MAX + MAX_LANG_IDS) * sizeof(int32_t)) + al(B * sizeof(int32_t));
     if (absorb) {
         const size_t Bd = B < 64 ? B : 64;
         ws += al((Bd * D.heads + ABSORB_QT_PAD) * d * e) + al(Bd * D.heads * d * e) +
@@ -1089,9 +1123,49 @@ int tw_encode(tw_model* m, const float* mel, int B, void* enc_out, int tap_layer
                                     : encode_impl<float>(m, mel, B, enc_out, tap_layer, tap_out, st);
 }
 
-static int check_decode_args(tw_model* m, int B, const int32_t* prompt, int P, const tw_rules* rules, int max_length) {
+// per-row prompts: host [B][P] ids, PROMPT_DETECT allowed at index 1 (then lang_ids are needed), the same SOT in every row
+static int check_prompt_rows(tw_model* m, int B, const tw_prompt_rows& rows, int P) {
     tw_ctx* ctx = m->ctx;
-    if (B <= 0 || B > m->desc.max_batch || !prompt || !rules) {
+    const int V = m->desc.vocab;
+    if (!rows.prompts || P < 1 || P > PROMPT_MAX) {
+        ctx->set_error(TW_E_INVALID, "decode: null prompt, or a prompt that is empty or longer than 24 tokens");
+        return TW_E_INVALID;
+    }
+    bool detect = false;
+    for (int b = 0; b < B; ++b)
+        for (int i = 0; i < P; ++i) {
+            const int t = rows.prompts[(size_t)b * P + i];
+            if (i == 1 && t == PROMPT_DETECT) { detect = true; continue; }
+            if (t < 0 || t >= V) {
+                ctx->set_error(TW_E_INVALID, "decode: prompt token out of range");
+                return TW_E_INVALID;
+            }
+            if (i == 0 && t != rows.prompts[0]) {
+                ctx->set_error(TW_E_INVALID, "decode: every row's prompt must start with the same token (SOT)");
+                return TW_E_INVALID;
+            }
+        }
+    if (rows.lang_ids || detect) {
+        if (!rows.lang_ids || rows.n_lang < 1 || rows.n_lang > MAX_LANG_IDS) {
+            ctx->set_error(TW_E_INVALID, "decode: language detection needs 1 .. 128 language ids");
+            return TW_E_INVALID;
+        }
+        for (int j = 0; j < rows.n_lang; ++j)
+            if (rows.lang_ids[j] < 0 || rows.lang_ids[j] >= V) {
+                ctx->set_error(TW_E_INVALID, "decode: language id out of range");
+                return TW_E_INVALID;
+            }
+    }
+    if (rows.out_lang && P < 2) {
+        ctx->set_error(TW_E_INVALID, "decode: out_lang needs a prompt with a language slot (P >= 2)");
+        return TW_E_INVALID;
+    }
+    return TW_OK;
+}
+
+static int check_decode_args(tw_model* m, int B, const tw_prompt_rows& rows, int P, const tw_rules* rules, int max_length) {
+    tw_ctx* ctx = m->ctx;
+    if (B <= 0 || B > m->desc.max_batch || !rules) {
         ctx->set_error(TW_E_INVALID, "decode: bad batch or null argument");
         return TW_E_INVALID;
     }
@@ -1101,16 +1175,24 @@ static int check_decode_args(tw_model* m, int B, const int32_t* prompt, int P, c
                                          std::to_string(m->desc.max_target) + ")");
         return TW_E_INVALID;
     }
-    for (int i = 0; i < P; ++i)
-        if (prompt[i] < 0 || prompt[i] >= m->desc.vocab) {
-            ctx->set_error(TW_E_INVALID, "decode: prompt token out of range");
-            return TW_E_INVALID;
-        }
-    return TW_OK;
+    return check_prompt_rows(m, B, rows, P);
 }
 
+// the single prompt of the original entry points, given to every row
+struct BroadcastPrompt {
+    std::vector<int32_t> ids;
+    tw_prompt_rows rows{};
+    BroadcastPrompt(const tw_model* m, const int32_t* prompt, int P, int B) {
+        if (m && prompt && P > 0 && P <= PROMPT_MAX && B > 0 && B <= m->desc.max_batch) {     // else the argument checks reject the call
+            ids.resize((size_t)B * P);
+            for (int b = 0; b < B; ++b) std::copy(prompt, prompt + P, ids.begin() + (size_t)b * P);
+            rows.prompts = ids.data();
+        }
+    }
+};
+
 // tw_decode_greedy after its argument checks; tw_debug_decode_taps adds residual taps
-static int decode_greedy_call(tw_model* m, const void* enc_out, int B, const int32_t* prompt, int P, const tw_rules* rules, int max_length,
+static int decode_greedy_call(tw_model* m, const void* enc_out, int B, const tw_prompt_rows& rows, int P, const tw_rules* rules, int max_length,
                               int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps,
                               cudaStream_t st, const DecodeTaps& taps) {
     RulesDev R;
@@ -1120,32 +1202,66 @@ static int decode_greedy_call(tw_model* m, const void* enc_out, int B, const int
     if (r != TW_OK) return r;
     cudaEventRecord(m->ev[3], st);
     r = m->desc.dtype == TW_BF16
-            ? decode_impl<__nv_bfloat16>(m, B, prompt, P, R, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps, st, taps)
-            : decode_impl<float>(m, B, prompt, P, R, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps, st, taps);
+            ? decode_impl<__nv_bfloat16>(m, B, rows, P, R, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps, st, taps)
+            : decode_impl<float>(m, B, rows, P, R, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps, st, taps);
     cudaEventRecord(m->ev[4], st);
     m->ev_valid[2] = m->ev_valid[3] = m->ev_valid[4] = true;
     m->ev_valid[0] = m->ev_valid[1] = m->ev_valid[6] = m->ev_valid[7] = false;
     return r;
 }
 
-int tw_decode_greedy(tw_model* m, const void* enc_out, int B, const int32_t* prompt, int P, const tw_rules* rules, int max_length,
-                     int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps,
-                     void* stream) {
+int tw_decode_greedy_rows(tw_model* m, const void* enc_out, int B, const tw_prompt_rows* rows, int P, const tw_rules* rules,
+                          int max_length, int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced, float* logits_tap,
+                          int tap_steps, void* stream) {
     if (!check_model(m, "tw_decode_greedy")) return TW_E_INVALID;
-    TW_CHECK(check_decode_args(m, B, prompt, P, rules, max_length));
+    if (!rows) {
+        m->ctx->set_error(TW_E_INVALID, "tw_decode_greedy_rows: null rows");
+        return TW_E_INVALID;
+    }
+    TW_CHECK(check_decode_args(m, B, *rows, P, rules, max_length));
     if (!enc_out || !out_tokens || !out_lengths) {
         m->ctx->set_error(TW_E_INVALID, "tw_decode_greedy: null buffer");
         return TW_E_INVALID;
     }
-    return decode_greedy_call(m, enc_out, B, prompt, P, rules, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps,
+    return decode_greedy_call(m, enc_out, B, *rows, P, rules, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps,
                               (cudaStream_t)stream, DecodeTaps{});
+}
+
+int tw_decode_greedy(tw_model* m, const void* enc_out, int B, const int32_t* prompt, int P, const tw_rules* rules, int max_length,
+                     int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps,
+                     void* stream) {
+    BroadcastPrompt bp(m, prompt, P, B);
+    return tw_decode_greedy_rows(m, enc_out, B, &bp.rows, P, rules, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps,
+                                 stream);
+}
+
+int tw_detect_language(tw_model* m, const void* enc_out, int B, const int32_t* lang_ids, int n_lang, int32_t* out_lang, void* stream) {
+    if (!check_model(m, "tw_detect_language")) return TW_E_INVALID;
+    tw_ctx* ctx = m->ctx;
+    if (B <= 0 || B > m->desc.max_batch || !enc_out || !out_lang) {
+        ctx->set_error(TW_E_INVALID, "tw_detect_language: bad batch (1..max_batch) or null buffer");
+        return TW_E_INVALID;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    // step 0 of a decode whose every row detects: prompt [SOT, detect], max_length 2 (one step, nothing generated, no graph)
+    std::vector<int32_t> prompts((size_t)B * 2);
+    for (int b = 0; b < B; ++b) { prompts[2 * b] = WHISPER_SOT; prompts[2 * b + 1] = PROMPT_DETECT; }
+    tw_prompt_rows rows{prompts.data(), lang_ids, n_lang, out_lang};
+    TW_CHECK(check_prompt_rows(m, B, rows, 2));
+    TW_CHECK(cross_kv_for_decode(m, enc_out, B, st));
+    RulesDev R{m->d_suppress, m->d_begin_suppress, -1, -1, -1, -1, -1};     // no token is selected
+    int r = m->desc.dtype == TW_BF16 ? decode_impl<__nv_bfloat16>(m, B, rows, 2, R, 2, m->d_out_tok, m->d_out_len, nullptr, nullptr, 0, st)
+                                     : decode_impl<float>(m, B, rows, 2, R, 2, m->d_out_tok, m->d_out_len, nullptr, nullptr, 0, st);
+    if (r == TW_OK) TW_CUDA_OK(ctx, cudaGetLastError());
+    return r;
 }
 
 int tw_debug_decode_taps(tw_model* m, const void* enc_out, int B, const int32_t* prompt, int P, const tw_rules* rules, int max_length,
                          int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced, float* logits_tap, int tap_steps,
                          float* layer_tap, int pos0, int n_pos, void* self_kv_out, int n_sms, void* stream) {
     if (!check_model(m, "tw_debug_decode_taps")) return TW_E_INVALID;
-    TW_CHECK(check_decode_args(m, B, prompt, P, rules, max_length));
+    BroadcastPrompt bp(m, prompt, P, B);
+    TW_CHECK(check_decode_args(m, B, bp.rows, P, rules, max_length));
     tw_ctx* ctx = m->ctx;
     if (!enc_out || !out_tokens || !out_lengths || (layer_tap && (pos0 < 0 || n_pos < 0 || pos0 + n_pos > max_length - 1)) || n_sms < 0) {
         ctx->set_error(TW_E_INVALID, "tw_debug_decode_taps: null buffer, tapped positions outside 0 .. max_length - 2 or n_sms < 0");
@@ -1160,7 +1276,7 @@ int tw_debug_decode_taps(tw_model* m, const void* enc_out, int B, const int32_t*
     const int sms_before = ctx->sm_count;
     const int da_before = decode_attention_set_sms(n_sms);
     if (n_sms > 0) ctx->sm_count = n_sms;
-    int r = decode_greedy_call(m, enc_out, B, prompt, P, rules, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps, st, taps);
+    int r = decode_greedy_call(m, enc_out, B, bp.rows, P, rules, max_length, out_tokens, out_lengths, forced, logits_tap, tap_steps, st, taps);
     decode_attention_set_sms(da_before);
     ctx->sm_count = sms_before;
     if (r != TW_OK || !self_kv_out) return r;
@@ -1220,8 +1336,20 @@ int tw_debug_decoder_logits_taps(tw_model* m, const void* enc_out, int B, const 
 
 int tw_transcribe_host(tw_model* m, const int16_t* pcm_host, const int32_t* n_valid_host, int B, const int32_t* prompt, int P,
                        const tw_rules* rules, int max_length, int32_t* out_tokens_host, int32_t* out_lengths_host, void* stream) {
+    BroadcastPrompt bp(m, prompt, P, B);
+    return tw_transcribe_host_rows(m, pcm_host, n_valid_host, B, &bp.rows, P, rules, max_length, out_tokens_host, out_lengths_host, stream);
+}
+
+int tw_transcribe_host_rows(tw_model* m, const int16_t* pcm_host, const int32_t* n_valid_host, int B, const tw_prompt_rows* rows_host,
+                            int P, const tw_rules* rules, int max_length, int32_t* out_tokens_host, int32_t* out_lengths_host, void* stream) {
     if (!check_model(m, "tw_transcribe_host")) return TW_E_INVALID;
-    TW_CHECK(check_decode_args(m, B, prompt, P, rules, max_length));
+    if (!rows_host) {
+        m->ctx->set_error(TW_E_INVALID, "tw_transcribe_host_rows: null rows");
+        return TW_E_INVALID;
+    }
+    TW_CHECK(check_decode_args(m, B, *rows_host, P, rules, max_length));
+    tw_prompt_rows rows = *rows_host;
+    rows.out_lang = rows_host->out_lang ? m->d_out_lang : nullptr;      // decoded on the device, copied to the host buffer below
     if (!pcm_host || !out_tokens_host || !out_lengths_host) {
         m->ctx->set_error(TW_E_INVALID, "tw_transcribe_host: null buffer");
         return TW_E_INVALID;
@@ -1252,11 +1380,13 @@ int tw_transcribe_host(tw_model* m, const int16_t* pcm_host, const int32_t* n_va
     if (r != TW_OK) return r;
     cudaEventRecord(m->ev[3], st);
     r = D.dtype == TW_BF16
-            ? decode_impl<__nv_bfloat16>(m, B, prompt, P, R, max_length, m->d_out_tok, m->d_out_len, nullptr, nullptr, 0, st)
-            : decode_impl<float>(m, B, prompt, P, R, max_length, m->d_out_tok, m->d_out_len, nullptr, nullptr, 0, st);
+            ? decode_impl<__nv_bfloat16>(m, B, rows, P, R, max_length, m->d_out_tok, m->d_out_len, nullptr, nullptr, 0, st)
+            : decode_impl<float>(m, B, rows, P, R, max_length, m->d_out_tok, m->d_out_len, nullptr, nullptr, 0, st);
     if (r != TW_OK) return r;
     TW_CUDA_OK(ctx, cudaMemcpyAsync(out_tokens_host, m->d_out_tok, (size_t)B * n_gen * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     TW_CUDA_OK(ctx, cudaMemcpyAsync(out_lengths_host, m->d_out_len, B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (rows.out_lang)
+        TW_CUDA_OK(ctx, cudaMemcpyAsync(rows_host->out_lang, m->d_out_lang, B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     cudaEventRecord(m->ev[4], st);
     TW_CUDA_OK(ctx, cudaStreamSynchronize(st));
     for (int i = 0; i < 5; ++i) m->ev_valid[i] = true;
@@ -1480,8 +1610,20 @@ int tw_pipeline_encode_at(tw_model* m, const int16_t* pcm, const int32_t* n_vali
 
 int tw_pipeline_decode(tw_model* m, int slot, int B, const int32_t* prompt, int P_len, const tw_rules* rules, int max_length,
                        int32_t* out_tokens_host, int32_t* out_lengths_host) {
+    BroadcastPrompt bp(m, prompt, P_len, B);
+    return tw_pipeline_decode_rows(m, slot, B, &bp.rows, P_len, rules, max_length, out_tokens_host, out_lengths_host);
+}
+
+int tw_pipeline_decode_rows(tw_model* m, int slot, int B, const tw_prompt_rows* rows_host, int P_len, const tw_rules* rules, int max_length,
+                            int32_t* out_tokens_host, int32_t* out_lengths_host) {
     if (!check_model(m, "tw_pipeline_decode")) return TW_E_INVALID;
-    TW_CHECK(check_decode_args(m, B, prompt, P_len, rules, max_length));
+    if (!rows_host) {
+        m->ctx->set_error(TW_E_INVALID, "tw_pipeline_decode_rows: null rows");
+        return TW_E_INVALID;
+    }
+    TW_CHECK(check_decode_args(m, B, *rows_host, P_len, rules, max_length));
+    tw_prompt_rows rows = *rows_host;
+    rows.out_lang = rows_host->out_lang ? m->d_out_lang : nullptr;      // decoded on the device, copied to the host buffer below
     tw_ctx* ctx = m->ctx;
     auto& P = m->pipe;
     if (!P.on || slot < 0 || slot > 1 || !out_tokens_host || !out_lengths_host) {
@@ -1505,14 +1647,16 @@ int tw_pipeline_decode(tw_model* m, int slot, int B, const int32_t* prompt, int 
     cudaEventRecord(P.dec_t0[slot], st);
     P.dec_timed[slot] = false;
     int r = D.dtype == TW_BF16
-                ? decode_impl<__nv_bfloat16>(m, B, prompt, P_len, R, max_length, m->d_out_tok, m->d_out_len, nullptr, nullptr, 0, st)
-                : decode_impl<float>(m, B, prompt, P_len, R, max_length, m->d_out_tok, m->d_out_len, nullptr, nullptr, 0, st);
+                ? decode_impl<__nv_bfloat16>(m, B, rows, P_len, R, max_length, m->d_out_tok, m->d_out_len, nullptr, nullptr, 0, st)
+                : decode_impl<float>(m, B, rows, P_len, R, max_length, m->d_out_tok, m->d_out_len, nullptr, nullptr, 0, st);
     P.in_decode = false;
     m->xkv = xkv_before;
     set_active_sms(m, sms_before);
     if (r != TW_OK) return r;
     TW_CUDA_OK(ctx, cudaMemcpyAsync(out_tokens_host, m->d_out_tok, (size_t)B * n_gen * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     TW_CUDA_OK(ctx, cudaMemcpyAsync(out_lengths_host, m->d_out_len, B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    if (rows.out_lang)
+        TW_CUDA_OK(ctx, cudaMemcpyAsync(rows_host->out_lang, m->d_out_lang, B * sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     cudaEventRecord(m->ev[4], st);
     cudaEventRecord(P.dec_t1[slot], st);
     P.dec_timed[slot] = true;
@@ -1839,8 +1983,20 @@ int tw_debug_set_row_budgets(tw_model* m, const int32_t* budgets_host, int n) {
 int tw_debug_select_steps(tw_model* m, const float* logits, int64_t ld_logits, int B, const int32_t* prompt, int P, const tw_rules* rules,
                           int max_length, const int32_t* row_budgets, const int32_t* forced, float* logits_tap, int tap_steps,
                           int32_t* out_tokens, int32_t* out_lengths, int32_t* n_active, int32_t* active, void* stream) {
+    BroadcastPrompt bp(m, prompt, P, B);
+    return tw_debug_select_steps_rows(m, logits, ld_logits, B, &bp.rows, P, rules, max_length, row_budgets, forced, logits_tap, tap_steps,
+                                      out_tokens, out_lengths, n_active, active, stream);
+}
+
+int tw_debug_select_steps_rows(tw_model* m, const float* logits, int64_t ld_logits, int B, const tw_prompt_rows* rows, int P,
+                               const tw_rules* rules, int max_length, const int32_t* row_budgets, const int32_t* forced, float* logits_tap,
+                               int tap_steps, int32_t* out_tokens, int32_t* out_lengths, int32_t* n_active, int32_t* active, void* stream) {
     if (!check_model(m, "tw_debug_select_steps")) return TW_E_INVALID;
-    TW_CHECK(check_decode_args(m, B, prompt, P, rules, max_length));
+    if (!rows) {
+        m->ctx->set_error(TW_E_INVALID, "tw_debug_select_steps_rows: null rows");
+        return TW_E_INVALID;
+    }
+    TW_CHECK(check_decode_args(m, B, *rows, P, rules, max_length));
     tw_ctx* ctx = m->ctx;
     const int V = m->desc.vocab, n_gen = max_length - P;
     if (!logits || !out_tokens || !out_lengths || ld_logits < V || (ld_logits % 4) || (reinterpret_cast<uintptr_t>(logits) & 15) ||
@@ -1855,12 +2011,14 @@ int tw_debug_select_steps(tw_model* m, const float* logits, int64_t ld_logits, i
     const bool budgets_before = m->row_budget_on;
     TW_CHECK(tw_debug_set_row_budgets(m, row_budgets, row_budgets ? B : 0));
     DecodeState S;
-    int r = begin_decode(m, B, prompt, P, max_length, out_lengths, logits_tap, tap_steps, st, &S);
+    int r = begin_decode(m, B, *rows, P, max_length, out_lengths, logits_tap, tap_steps, st, &S);
     // the decode loop of decode_impl with the logits of generated step g read from logits + g * B * ld_logits instead of the model
+    // (prompt steps read those of step 0; so does the language pick of position 0)
     for (int pos = 0; r == TW_OK && pos < max_length - 1; ++pos) {
         const int g = pos - (P - 1);
-        select_tokens(logits + (int64_t)(g > 0 ? g : 0) * B * ld_logits, ld_logits, V, B, m->d_step, R, S, out_tokens, out_lengths, forced,
-                      logits_tap, st);
+        const float* lg = logits + (int64_t)(g > 0 ? g : 0) * B * ld_logits;
+        if (pos == 0 && m->pick_now) pick_language(lg, ld_logits, B, m->d_lang_ids, m->n_lang_now, S, rows->out_lang, st);
+        else select_tokens(lg, ld_logits, V, B, m->d_step, R, S, out_tokens, out_lengths, forced, logits_tap, st);
         advance_step(m->d_step, S, B, st);
         ctx->launches += 2;
         if (g >= 0 && n_active && cudaMemcpyAsync(n_active + g, S.n_active, sizeof(int32_t), cudaMemcpyDeviceToDevice, st) != cudaSuccess) r = TW_E_CUDA;

@@ -71,7 +71,7 @@ select_tokens_kernel(const float* __restrict__ logits, int64_t ld_logits, int V,
     const int pos = d_step[STEP_POS], P = d_step[STEP_P], out_stride = d_step[STEP_STRIDE];
     const int gen_index = pos - (P - 1);
     if (gen_index < 0) {                       // still consuming the forced prompt: feed the next prompt token
-        if (threadIdx.x == 0) S.cur_tok[b] = d_step[STEP_PROMPT + pos + 1];
+        if (threadIdx.x == 0) S.cur_tok[b] = S.prompt[b * PROMPT_MAX + pos + 1];
         return;
     }
     if (gen_index >= out_stride) return;
@@ -211,6 +211,42 @@ void select_tokens(const float* logits, int64_t ld_logits, int V, int B, const i
                    int32_t* out_tokens, int32_t* out_lengths, const int32_t* forced, float* logits_tap, cudaStream_t stream) {
     launch_k(select_tokens_kernel, dim3(B), dim3(SEL_THREADS), 0, stream, logits, ld_logits, V, d_step, rules, st, out_tokens, out_lengths, forced,
              logits_tap);
+}
+
+// Language detection (HF WhisperGenerationMixin.detect_language, generation_whisper.py:1610-1673): the logits of the step fed SOT,
+// every id outside lang_ids set to -inf, argmax.  One warp per row over the <= MAX_LANG_IDS candidates.
+constexpr int PICK_WARPS = 4;
+__global__ void __launch_bounds__(PICK_WARPS * 32)
+pick_language_kernel(const float* __restrict__ logits, int64_t ld_logits, int B, const int32_t* __restrict__ lang_ids, int n_lang,
+                     DecodeState S, int32_t* __restrict__ out_lang) {
+    pdl_trigger();
+    pdl_wait();
+    const int b = blockIdx.x * PICK_WARPS + (threadIdx.x >> 5), lane = threadIdx.x & 31;
+    if (b >= B) return;
+    int32_t* slot = S.prompt + (int64_t)b * PROMPT_MAX + 1;
+    int tok = *slot;
+    if (tok == PROMPT_DETECT) {
+        const float* row = logits + (int64_t)b * ld_logits;
+        Best best = {-INFINITY, 0x7fffffff};
+        for (int j = lane; j < n_lang; j += 32) {
+            const int id = lang_ids[j];
+            best = better(best, Best{row[id], id});
+        }
+        best = warp_best(best);
+        // all candidates -inf: the masked row is -inf everywhere and torch.argmax returns index 0
+        tok = best.v == -INFINITY ? 0 : best.i;
+    }
+    if (lane == 0) {
+        *slot = tok;
+        S.cur_tok[b] = tok;
+        if (out_lang) out_lang[b] = tok;
+    }
+}
+
+void pick_language(const float* logits, int64_t ld_logits, int B, const int32_t* lang_ids, int n_lang, const DecodeState& st,
+                   int32_t* out_lang, cudaStream_t stream) {
+    launch_k(pick_language_kernel, dim3(ceil_div(B, PICK_WARPS)), dim3(PICK_WARPS * 32), 0, stream, logits, ld_logits, B, lang_ids, n_lang,
+             st, out_lang);
 }
 
 __global__ void decode_state_init_kernel(DecodeState S, int B, int first_tok) {

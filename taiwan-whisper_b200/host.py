@@ -156,6 +156,59 @@ def greedy_decode(handle: int, enc_out: torch.Tensor, prompt: Sequence[int], max
     return (toks, lens, tap) if tap_steps else (toks, lens)
 
 
+def greedy_decode_rows(handle: int, enc_out: torch.Tensor, prompts: Sequence[Sequence[int]], lang_ids: Optional[Sequence[int]],
+                       max_length: int, suppress: Sequence[int], begin_suppress: Sequence[int], eos: int, pad: int, timestamp_begin: int,
+                       no_timestamps: int, max_initial_ts: int):
+    """greedy_decode with one forced prompt per row (tw_decode_greedy_rows): prompts [B][P], lib.PROMPT_DETECT at index 1 = detect
+    that row's language in step 0 among lang_ids.  Returns (tokens int32 [B, max_length - P], lengths int32 [B], languages int32 [B]:
+    token 1 of every row's prompt as decoded)."""
+    d = model_desc(handle)
+    B = enc_out.shape[0]
+    if len(prompts) != B:
+        raise ValueError(f"{len(prompts)} prompts for {B} rows")
+    n_gen = max_length - len(prompts[0])
+    if n_gen <= 0 or max_length > d.max_target:
+        raise ValueError(f"The length of the prompt ({len(prompts[0])}) plus the new tokens must fit max_length "
+                         f"<= max_target_positions ({d.max_target}); got max_length={max_length}")
+    dev = _dev_index(enc_out.device)
+    ctx = _lib.Context.get(dev)
+    enc_out = enc_out.to(_TW2TORCH[d.dtype]).contiguous()
+    toks = torch.empty((B, n_gen), dtype=torch.int32, device=enc_out.device)
+    lens = torch.empty((B,), dtype=torch.int32, device=enc_out.device)
+    detect = any(p[1] == _lib.PROMPT_DETECT for p in prompts if len(p) > 1)
+    langs = torch.empty((B,), dtype=torch.int32, device=enc_out.device) if detect else None
+    rows, keep_rows, P = _lib.make_prompt_rows(prompts, lang_ids if detect else None, langs.data_ptr() if detect else None)
+    rules, keep = _lib.make_rules(list(suppress), list(begin_suppress), int(eos), int(pad),
+                                  None if timestamp_begin is None or timestamp_begin < 0 else int(timestamp_begin),
+                                  int(no_timestamps), None if max_initial_ts is None or max_initial_ts < 0 else int(max_initial_ts))
+    with torch.cuda.device(dev):
+        ctx.check(ctx.lib.tw_decode_greedy_rows(C.c_void_p(handle), enc_out.data_ptr(), B, C.byref(rows), P, C.byref(rules), max_length,
+                                                toks.data_ptr(), lens.data_ptr(), None, None, 0, _stream_ptr(enc_out.device)))
+    del keep, keep_rows
+    if not detect:       # every language was given: nothing to read back
+        langs = torch.tensor([p[1] if len(p) > 1 else -1 for p in prompts], dtype=torch.int32, device=enc_out.device)
+    return toks, lens, langs
+
+
+def detect_language(handle: int, enc_out: torch.Tensor, lang_ids) -> torch.Tensor:
+    """enc_out [B, 1500, d] (cuda) -> int32 [B]: the language id of every row (tw_detect_language: the logits of the step fed
+    <|startoftranscript|>, masked to lang_ids, argmax — HF WhisperGenerationMixin.detect_language)."""
+    d = model_desc(handle)
+    if enc_out.dim() != 3 or enc_out.shape[1:] != (1500, d.d_model):
+        raise ValueError(f"encoder output must be [B, 1500, {d.d_model}], got {tuple(enc_out.shape)}")
+    ids = [int(t) for t in (lang_ids.tolist() if torch.is_tensor(lang_ids) else lang_ids)]
+    dev = _dev_index(enc_out.device)
+    ctx = _lib.Context.get(dev)
+    enc_out = enc_out.to(_TW2TORCH[d.dtype]).contiguous()
+    B = enc_out.shape[0]
+    out = torch.empty((B,), dtype=torch.int32, device=enc_out.device)
+    arr = (C.c_int32 * max(1, len(ids)))(*ids)
+    with torch.cuda.device(dev):
+        ctx.check(ctx.lib.tw_detect_language(C.c_void_p(handle), enc_out.data_ptr(), B, arr, len(ids), out.data_ptr(),
+                                             _stream_ptr(enc_out.device)))
+    return out
+
+
 def decoder_logits(handle: int, enc_out: torch.Tensor, decoder_input_ids: torch.Tensor) -> torch.Tensor:
     """enc_out [B,1500,d] + decoder_input_ids [B,T] -> fp32 logits [B,T,V] of every position in ONE batched decoder pass
     (tw_decoder_logits).  The returned tensor is a view whose row pitch is V rounded up to 4 floats."""
@@ -183,7 +236,7 @@ def decoder_logits(handle: int, enc_out: torch.Tensor, decoder_input_ids: torch.
 
 
 def _register_torch_ops():
-    """torch.ops.twb200.{log_mel, model_create, model_free, encoder_forward, greedy_generate, decoder_logits}: operator
+    """torch.ops.twb200.{log_mel, model_create, model_free, encoder_forward, greedy_generate, decoder_logits, detect_language}: operator
     wrappers over the C ABI (CUDA tensors only, current stream).  A model is addressed by its `tw_model*` passed as an int —
     the value model_create returns — so the ops need no Python-side object (SURVEY §8b)."""
     try:
@@ -238,6 +291,14 @@ def _register_torch_ops():
     def _(handle, enc_out, decoder_input_ids):
         d = model_desc(handle)
         return enc_out.new_empty((decoder_input_ids.shape[0], decoder_input_ids.shape[1], d.vocab), dtype=torch.float32)
+
+    @custom_op("twb200::detect_language", mutates_args=())
+    def _op_detect_language(handle: int, enc_out: torch.Tensor, lang_ids: torch.Tensor) -> torch.Tensor:
+        return detect_language(handle, enc_out, lang_ids)
+
+    @_op_detect_language.register_fake
+    def _(handle, enc_out, lang_ids):
+        return enc_out.new_empty((enc_out.shape[0],), dtype=torch.int32)
 
 
 # --------------------------------------------------------------------------------------------
@@ -478,39 +539,112 @@ class B200WhisperForConditionalGeneration:
 
     # ---- generation config plumbing (generation_whisper.py:1455-1608, :1774-1812)
     def _init_tokens(self, language, task, return_timestamps):
+        """The one forced prompt of a call that names a single language (or of an English-only checkpoint)."""
+        if self._is_multilingual() and (language is None or isinstance(language, (list, tuple))):
+            raise NotImplementedError("language=None (detection) and language lists give every row its own prompt: "
+                                      "_row_prompts(language, task, return_timestamps, batch_size) builds them")
+        return self._row_prompts(language, task, return_timestamps, 1)[0]
+
+    def _is_multilingual(self):
         gc = self.generation_config
         is_multi = getattr(gc, "is_multilingual", None)
         if is_multi is None or not hasattr(gc, "lang_to_id") or not hasattr(gc, "task_to_id"):
             raise ValueError("The generation config is outdated: it needs `is_multilingual`, `lang_to_id`, `task_to_id` "
                              "and `no_timestamps_token_id` (as generation_config.json of the released checkpoints has).")
-        toks = [self.config.decoder_start_token_id]
-        if not is_multi:
+        return bool(is_multi)
+
+    def _row_prompts(self, language, task, return_timestamps, batch_size):
+        """The forced prompt of every row, as HF's _retrieve_init_tokens builds them (generation_whisper.py:1455-1608): one
+        language for all rows, a list with one language per row, or language=None — detection, marked by lib.PROMPT_DETECT at
+        index 1, where step 0 of the decode writes the detected id.  Detection follows HF: no task token unless `task` is given
+        or `forced_decoder_ids` (generation config, else model config) force one, and a language those force is not detected."""
+        gc = self.generation_config
+        if not self._is_multilingual():
             if language is not None or task is not None:
                 raise ValueError("Cannot specify `task` or `language` for an English-only model.")
+            toks = [self.config.decoder_start_token_id]
+            if not return_timestamps:
+                toks.append(gc.no_timestamps_token_id)
+            return [toks] * batch_size
+        if isinstance(language, (list, tuple)):
+            if any(l is None for l in language):
+                raise TypeError(
+                    "Expected `language` to be `None`, a single string (e.g. `'en'`), or a list of strings with "
+                    "length equal to the batch size (e.g. `('en', 'fr')` for a batch size of 2). Got a list "
+                    "containing `None`.")
+            if len(language) != batch_size:
+                raise ValueError(
+                    "When passing a list of languages, the length of the list must match the batch size. "
+                    f"Expected length of {batch_size}, but got {len(language)} languages.")
+            return [self._lang_prompt(l, task, return_timestamps) for l in language]
+        if language is not None:
+            return [self._lang_prompt(language, task, return_timestamps)] * batch_size
+        return [self._detect_prompt(task, return_timestamps)] * batch_size
+
+    def _detect_prompt(self, task, return_timestamps):
+        """_retrieve_init_tokens with language=None (generation_whisper.py:1484-1606), the language slot left to detection."""
+        gc = self.generation_config
+        toks = [self.config.decoder_start_token_id]
+        if task is None:
+            forced = getattr(gc, "forced_decoder_ids", None)
+            if forced is None:
+                forced = getattr(self.config, "forced_decoder_ids", None)
+            if forced is not None and forced[0][0] == 1:
+                i = 1
+                while len(forced) > 0 and forced[0][0] == i:
+                    toks.append(forced[0][1])
+                    forced = forced[1:]
+                    i += 1
+                if len(forced) > 0:
+                    raise ValueError(
+                        f"You are using token ids in `forced_decoder_ids` that do not seem to correctly follow "
+                        f"the prompt pattern of Whisper. Make sure that {forced} has an entry for all "
+                        f"indices >= 1 and < {forced[0][0]}.")
+        if len(toks) <= 1:
+            toks.append(_lib.PROMPT_DETECT)
+        elif toks[1] is None:
+            toks[1] = _lib.PROMPT_DETECT
+        if task is not None:
+            if task not in gc.task_to_id:
+                raise ValueError(f"The `{task}` task is not supported. The task should be one of `{list(gc.task_to_id)}`")
+            toks.append(gc.task_to_id[task])
+        if not return_timestamps and toks[-1] != gc.no_timestamps_token_id:
+            toks.append(gc.no_timestamps_token_id)
+        elif return_timestamps and toks[-1] == gc.no_timestamps_token_id:
+            toks = toks[:-1]
+        return [t for t in toks if t is not None]
+
+    def _lang_prompt(self, language, task, return_timestamps):
+        """One prompt with a given language (a code, "<|code|>" or a name); the task defaults to transcribe."""
+        gc = self.generation_config
+        toks = [self.config.decoder_start_token_id]
+        lang = str(language).lower()
+        if lang in gc.lang_to_id:
+            lang_tok = lang
+        elif f"<|{lang}|>" in gc.lang_to_id:
+            lang_tok = f"<|{lang}|>"
+        elif lang in _LANG_NAMES and f"<|{_LANG_NAMES[lang]}|>" in gc.lang_to_id:
+            lang_tok = f"<|{_LANG_NAMES[lang]}|>"
         else:
-            if language is None:
-                # HF runs language detection here (generation_whisper.py:1530-1560); the reference always forwards
-                # data_args.language / 'zh'.  Guessing a language would silently mislabel a corpus.
-                raise NotImplementedError("language=None on a multilingual checkpoint needs language detection, which the "
-                                          "B200 path does not implement: pass language='zh' (or another code) explicitly")
-            lang = str(language).lower()
-            if lang in gc.lang_to_id:
-                lang_tok = lang
-            elif f"<|{lang}|>" in gc.lang_to_id:
-                lang_tok = f"<|{lang}|>"
-            elif lang in _LANG_NAMES and f"<|{_LANG_NAMES[lang]}|>" in gc.lang_to_id:
-                lang_tok = f"<|{_LANG_NAMES[lang]}|>"
-            else:
-                raise ValueError(f"Unsupported language: {language}. Language should be one of: "
-                                 f"{sorted(gc.lang_to_id.keys())[:8]}...")
-            toks.append(gc.lang_to_id[lang_tok])
-            t = "transcribe" if task is None else task
-            if t not in gc.task_to_id:
-                raise ValueError(f"The `{t}` task is not supported. The task should be one of `{list(gc.task_to_id)}`")
-            toks.append(gc.task_to_id[t])
+            raise ValueError(f"Unsupported language: {language}. Language should be one of: "
+                             f"{sorted(gc.lang_to_id.keys())[:8]}...")
+        toks.append(gc.lang_to_id[lang_tok])
+        t = "transcribe" if task is None else task
+        if t not in gc.task_to_id:
+            raise ValueError(f"The `{t}` task is not supported. The task should be one of `{list(gc.task_to_id)}`")
+        toks.append(gc.task_to_id[t])
         if not return_timestamps:
             toks.append(gc.no_timestamps_token_id)
         return toks
+
+    def _lang_ids(self):
+        """The ids language detection chooses among: the values of generation_config.lang_to_id."""
+        return sorted(int(v) for v in self.generation_config.lang_to_id.values())
+
+    @staticmethod
+    def _resolved(prompts, langs):
+        """prompts with every detection slot replaced by the row's decoded language (langs: int sequence [B])."""
+        return [[int(langs[b]) if (i == 1 and t == _lib.PROMPT_DETECT) else t for i, t in enumerate(p)] for b, p in enumerate(prompts)]
 
     def _rules(self, return_timestamps):
         gc = self.generation_config
@@ -535,6 +669,34 @@ class B200WhisperForConditionalGeneration:
         return greedy_decode(self.handle, enc_out.to(self.device), list(prompt), max_length, r["suppress"], r["begin_suppress"],
                              r["eos"], r["pad"], -1 if r["timestamp_begin"] is None else r["timestamp_begin"], r["no_timestamps"],
                              -1 if r["max_initial_ts"] is None else r["max_initial_ts"], forced=forced, tap_steps=tap_steps)
+
+    def decode_rows(self, enc_out: torch.Tensor, prompts, max_length: int, timestamps: bool):
+        """decode with one prompt per row (_row_prompts): returns (tokens, lengths, languages int32 [B]), the languages detected
+        in step 0 for rows whose prompt asks for it, the given ones elsewhere."""
+        r = self._rules(timestamps)
+        return greedy_decode_rows(self.handle, enc_out.to(self.device), prompts, self._lang_ids(), max_length, r["suppress"],
+                                  r["begin_suppress"], r["eos"], r["pad"], -1 if r["timestamp_begin"] is None else r["timestamp_begin"],
+                                  r["no_timestamps"], -1 if r["max_initial_ts"] is None else r["max_initial_ts"])
+
+    @torch.no_grad()
+    def detect_language(self, input_features=None, encoder_outputs=None, generation_config=None, num_segment_frames: int = N_FRAMES):
+        """WhisperGenerationMixin.detect_language (generation_whisper.py:1610-1673): LongTensor [B] of language ids, from log-mel
+        input_features [B, n_mel, >= 3000] (the first 3000 frames) or encoder_outputs ([B, 1500, d], a tuple or an object with
+        last_hidden_state).  Step 0 of a decode fed <|startoftranscript|>, its logits masked to lang_to_id, argmax."""
+        if input_features is None and encoder_outputs is None:
+            raise ValueError("You have to specify either `input_features` or `encoder_outputs`")
+        elif input_features is not None and encoder_outputs is not None:
+            raise ValueError("Make sure to specify only one of `input_features` or `encoder_outputs` - not both!")
+        lang_ids = self._lang_ids()
+        if input_features is not None:
+            feats = torch.as_tensor(input_features)[:, :, :num_segment_frames]
+            encs = [self.encode(feats[s:s + self.max_batch].to(self.device).float()) for s in range(0, feats.shape[0], self.max_batch)]
+        else:
+            enc = encoder_outputs[0] if isinstance(encoder_outputs, (tuple, list)) else getattr(encoder_outputs, "last_hidden_state",
+                                                                                                 encoder_outputs)
+            enc = torch.as_tensor(enc).to(self.device)
+            encs = [enc[s:s + self.max_batch] for s in range(0, enc.shape[0], self.max_batch)]
+        return torch.cat([detect_language(self.handle, e, lang_ids) for e in encs]).long()
 
     def decoder_logits(self, enc_out: torch.Tensor, decoder_input_ids: torch.Tensor) -> torch.Tensor:
         """enc_out [B,1500,d] + decoder_input_ids [B,T] -> fp32 logits [B,T,V] of every position in ONE batched decoder pass."""
@@ -581,17 +743,19 @@ class B200WhisperForConditionalGeneration:
 
     def transcribe_pcm(self, pcm_host: torch.Tensor, max_length: int, return_timestamps: bool = False, language="zh",
                        task="transcribe", n_valid: Optional[torch.Tensor] = None, out_tokens: Optional[torch.Tensor] = None,
-                       out_lengths: Optional[torch.Tensor] = None):
+                       out_lengths: Optional[torch.Tensor] = None, return_languages: bool = False):
         """Whole path from HOST int16 PCM [B, 480000] (pinned for async copies) to HOST token ids:
-        one C-ABI call = fe(...) + generate(...) of the reference."""
+        one C-ABI call = fe(...) + generate(...) of the reference.  `language`: one for every row, a list with one per row, or
+        None — each row's language is detected in the decode's first step.  return_languages: also return the host int32 [B]
+        language ids the rows were decoded with."""
         if pcm_host.dtype != torch.int16 or pcm_host.dim() != 2 or pcm_host.shape[1] != N_SAMPLES or pcm_host.is_cuda:
             raise ValueError("transcribe_pcm expects a host int16 tensor [B, 480000]")
         pcm_host = pcm_host.contiguous()
         B = pcm_host.shape[0]
         if B > self.max_batch:
             raise ValueError(f"batch {B} > max_batch {self.max_batch}")
-        prompt = self._init_tokens(language, task, return_timestamps)
-        n_gen = max_length - len(prompt)
+        prompts = self._row_prompts(language, task, return_timestamps, B)
+        n_gen = max_length - len(prompts[0])
         if n_gen <= 0 or max_length > self.shape.max_target:
             raise ValueError("max_length must exceed the prompt and fit max_target_positions")
         if out_tokens is None:
@@ -600,14 +764,23 @@ class B200WhisperForConditionalGeneration:
         r = self._rules(return_timestamps)
         rules, keep = _lib.make_rules(r["suppress"], r["begin_suppress"], r["eos"], r["pad"], r["timestamp_begin"],
                                       r["no_timestamps"], r["max_initial_ts"])
-        p = (C.c_int32 * len(prompt))(*prompt)
+        rows, keep_rows, langs = self._prompt_rows(prompts, return_languages)
         nv = n_valid.contiguous().data_ptr() if n_valid is not None else None
         with torch.cuda.device(self.device):
-            self.ctx.check(self.ctx.lib.tw_transcribe_host(
-                C.c_void_p(self.handle), pcm_host.data_ptr(), nv, B, p, len(prompt), C.byref(rules), max_length, out_tokens.data_ptr(),
-                out_lengths.data_ptr(), _stream_ptr(self.device)))
-        del keep
-        return out_tokens, out_lengths
+            self.ctx.check(self.ctx.lib.tw_transcribe_host_rows(
+                C.c_void_p(self.handle), pcm_host.data_ptr(), nv, B, C.byref(rows), len(prompts[0]), C.byref(rules), max_length,
+                out_tokens.data_ptr(), out_lengths.data_ptr(), _stream_ptr(self.device)))
+        del keep, keep_rows
+        return (out_tokens, out_lengths, langs) if return_languages else (out_tokens, out_lengths)
+
+    def _prompt_rows(self, prompts, want_languages: bool):
+        """(PromptRows, keepalive, host int32 [B] language buffer or None) for the host-output entry points: the language ids go
+        along when a row detects, the language buffer when a row detects or the caller wants the languages."""
+        detect = any(len(p) > 1 and p[1] == _lib.PROMPT_DETECT for p in prompts)
+        langs = torch.empty((len(prompts),), dtype=torch.int32) if (detect or want_languages) else None
+        rows, keep, _ = _lib.make_prompt_rows(prompts, self._lang_ids() if detect else None,
+                                              langs.data_ptr() if langs is not None else None)
+        return rows, keep, langs
 
     # ------------------------------------------------------------------ pipelined batch loop (tw_pipeline_*)
     def enable_pipeline(self, n_enc_sms: int = 24):
@@ -646,7 +819,7 @@ class B200WhisperForConditionalGeneration:
         return max(16, min(want, (n_dev // 2) // 8 * 8))
 
     def transcribe_batches(self, batches, max_length: int, return_timestamps: bool = False, language="zh", task="transcribe",
-                           merge: int = 1, auto_sms: bool = False):
+                           merge: int = 1, auto_sms: bool = False, return_languages: bool = False):
         """The reference's batch loop (ref training/run_pseudo_labelling.py:915-918) as a generator: yields (tokens, lengths) — pinned
         host int32 tensors [B, max_length - P] / [B] — for every int16 PCM batch [B, 480000] of `batches` (pinned host or device
         tensors), in order.  While batch i decodes, batch i+1 is already in its log-mel / encoder / cross-K/V stage on the other SM
@@ -662,41 +835,49 @@ class B200WhisperForConditionalGeneration:
         `auto_sms=True` re-balances the two partitions while the loop runs: after every group the stage times of the last one
         (tw_pipeline_stage_ms) are compared and the encoder partition is resized when stage 1 has become the bottleneck or idles
         more than a quarter of the time (`_balanced_sms`).  Full-length rows keep the decode busy ~7x longer than stage 1 needs the
-        GPU; rows that end early (real audio) shift the balance towards stage 1 — the right split depends on the data."""
+        GPU; rows that end early (real audio) shift the balance towards stage 1 — the right split depends on the data.
+
+        `language`: one language (or None: every row's is detected in the decode's first step) for all rows, or a list with one
+        entry per batch of `batches` — a language, None or a list with one language per row of that batch.  Merged groups mix rows
+        of different languages freely.  return_languages: yield (tokens, lengths, languages), languages the host int32 [B] ids
+        the rows were decoded with."""
         if not getattr(self, "pipeline_sms", None):
             raise RuntimeError("transcribe_batches needs enable_pipeline() first")
         if merge < 1:
             raise ValueError("merge must be >= 1")
-        prompt = self._init_tokens(language, task, return_timestamps)
-        n_gen = max_length - len(prompt)
-        if n_gen <= 0 or max_length > self.shape.max_target:
-            raise ValueError("max_length must exceed the prompt and fit max_target_positions")
+        per_batch = isinstance(language, (list, tuple))
+
+        def batch_prompts(k, n):
+            lang = (language[k] if k < len(language) else None) if per_batch else language
+            return self._row_prompts(lang, task, return_timestamps, n)
+
         r = self._rules(return_timestamps)
         rules, keep = _lib.make_rules(r["suppress"], r["begin_suppress"], r["eos"], r["pad"], r["timestamp_begin"],
                                       r["no_timestamps"], r["max_initial_ts"])
-        p = (C.c_int32 * len(prompt))(*prompt)
         lib, h = self.ctx.lib, C.c_void_p(self.handle)
-        it = iter(batches)
+        it = enumerate(batches)
         pending = []                 # a batch that did not fit the current group
 
         def encode_group(slot):
             """Stage 1 of the next `merge` batches (fewer at the end of the loop, or when the next batch would not fit max_batch)
             into `slot`; returns the row count of each and keeps the PCM tensors alive until their decode has returned."""
-            sizes, alive = [], []
+            sizes, alive, prompts = [], [], []
             while len(sizes) < merge:
-                pcm = pending.pop() if pending else next(it, None)
-                if pcm is None:
+                kp = pending.pop() if pending else next(it, None)
+                if kp is None:
                     break
+                k, pcm = kp
                 if pcm.dtype != torch.int16 or pcm.dim() != 2 or pcm.shape[1] != N_SAMPLES or pcm.shape[0] > self.max_batch or pcm.shape[0] == 0:
                     raise ValueError("transcribe_batches expects int16 tensors [1 <= B <= max_batch, 480000]")
                 if sum(sizes) + pcm.shape[0] > self.max_batch:
-                    pending.append(pcm)                # opens the next group
+                    pending.append(kp)                 # opens the next group
                     break
                 pcm = pcm.contiguous()
+                prompts += batch_prompts(k, pcm.shape[0])
                 self.ctx.check(lib.tw_pipeline_encode_at(h, pcm.data_ptr(), None, pcm.shape[0], slot, sum(sizes)))
                 sizes.append(pcm.shape[0])
                 alive.append(pcm)
-            return (sizes, alive) if sizes else None
+            return (sizes, alive, prompts) if sizes else None
 
         with torch.cuda.device(self.device):
             cur = encode_group(0)
@@ -704,10 +885,16 @@ class B200WhisperForConditionalGeneration:
             while cur is not None:
                 nxt = encode_group((i + 1) & 1)
                 B = sum(cur[0])
+                P = len(cur[2][0])
+                n_gen = max_length - P
+                if n_gen <= 0 or max_length > self.shape.max_target:
+                    raise ValueError("max_length must exceed the prompt and fit max_target_positions")
                 out_tokens = torch.empty((B, n_gen), dtype=torch.int32).pin_memory()
                 out_lengths = torch.empty((B,), dtype=torch.int32).pin_memory()
-                self.ctx.check(lib.tw_pipeline_decode(h, i & 1, B, p, len(prompt), C.byref(rules), max_length, out_tokens.data_ptr(),
-                                                      out_lengths.data_ptr()))
+                rows, keep_rows, langs = self._prompt_rows(cur[2], return_languages)
+                self.ctx.check(lib.tw_pipeline_decode_rows(h, i & 1, B, C.byref(rows), P, C.byref(rules), max_length,
+                                                           out_tokens.data_ptr(), out_lengths.data_ptr()))
+                del keep_rows
                 if auto_sms and nxt is not None and sum(nxt[0]) == B:
                     # stage 1 of the NEXT group ran beside this decode: both times are of the same concurrent interval
                     t_enc, _ = self.pipeline_stage_ms((i + 1) & 1)
@@ -723,7 +910,10 @@ class B200WhisperForConditionalGeneration:
                         self.sms_history = getattr(self, "sms_history", []) + [self.pipeline_sms]
                 b0 = 0
                 for n in cur[0]:
-                    yield out_tokens[b0:b0 + n], out_lengths[b0:b0 + n]
+                    if return_languages:
+                        yield out_tokens[b0:b0 + n], out_lengths[b0:b0 + n], langs[b0:b0 + n]
+                    else:
+                        yield out_tokens[b0:b0 + n], out_lengths[b0:b0 + n]
                     b0 += n
                 cur = nxt
                 i += 1
@@ -756,7 +946,7 @@ class B200WhisperForConditionalGeneration:
     # ---- the reference's call
     @torch.no_grad()
     def generate(self, input_features=None, *, max_length: Optional[int] = None, max_new_tokens: Optional[int] = None,
-                 num_beams: int = 1, return_timestamps: Optional[bool] = None, language: Optional[str] = None,
+                 num_beams: int = 1, return_timestamps: Optional[bool] = None, language=None,
                  task: Optional[str] = None, attention_mask=None, return_prompt: Optional[bool] = None,
                  seek_loop: Optional[bool] = None, **kwargs):
         """ref: training/run_pseudo_labelling.py:864-876,917-918; prefiltering/validator_inference.py:41-47,78.
@@ -766,7 +956,10 @@ class B200WhisperForConditionalGeneration:
         ids and therefore needs it.  `seek_loop` (default: False under "4.45", True under "5.x"): with
         return_timestamps=True, run the 5.x seek loop around the window primitive — split at consecutive timestamp
         tokens, advance to the last predicted timestamp, re-encode the zero-padded remainder (generation_whisper.py:
-        785-900, 1976-2073) — or decode each window exactly once (short-form behaviour of 4.45)."""
+        785-900, 1976-2073) — or decode each window exactly once (short-form behaviour of 4.45).
+        `language`: one language for every row, a list with one per row, or None on a multilingual checkpoint — each row's
+        language is detected (detect_language) in the first step of its decode, with HF's prompts (_row_prompts); the seek loop
+        detects on a window's first pass and keeps that language for the rest of the window."""
         if return_prompt is None:
             return_prompt = self.output_layout == "4.45"
         if seek_loop is None:
@@ -786,24 +979,25 @@ class B200WhisperForConditionalGeneration:
             raise ValueError(f"Whisper expects the mel input features to be of length {N_FRAMES}, but found "
                              f"{feats.shape[-1]}. Make sure to pad the input mel features to {N_FRAMES}.")
         ts = bool(return_timestamps) if return_timestamps is not None else False
-        prompt = self._init_tokens(language, task, ts)
+        prompts = self._row_prompts(language, task, ts, feats.shape[0])
         if max_length is None:
             if max_new_tokens is not None:
-                max_length = len(prompt) + max_new_tokens
+                max_length = len(prompts[0]) + max_new_tokens
             else:
                 max_length = getattr(self.generation_config, "max_length", None) or self.shape.max_target
         if max_length > self.shape.max_target:
             raise ValueError(f"max_length={max_length} exceeds max_target_positions={self.shape.max_target}")
         pad = self._rules(ts)["pad"]
         if ts and seek_loop:
-            return self._generate_seek_loop(feats, prompt, max_length, pad, return_prompt)
-        rows, lens_all = [], []
+            return self._generate_seek_loop(feats, prompts, max_length, pad, return_prompt)
+        rows, lens_all, langs = [], [], []
         for s in range(0, feats.shape[0], self.max_batch):
             chunk = feats[s:s + self.max_batch]
             enc = self.encode(chunk.to(self.device).float())
-            toks, lens = self.decode(enc, prompt, max_length, ts)
+            toks, lens, lg = self.decode_rows(enc, prompts[s:s + self.max_batch], max_length, ts)
             rows.append(toks)
             lens_all.append(lens)
+            langs += lg.tolist()
         toks = torch.cat(rows).long()
         lens = torch.cat(lens_all).long()
         L = int(lens.max().item()) if lens.numel() else 0
@@ -811,15 +1005,16 @@ class B200WhisperForConditionalGeneration:
         ar = torch.arange(L, device=toks.device)[None, :]
         toks = torch.where(ar < lens[:, None], toks, torch.full_like(toks, pad))
         if return_prompt:
-            toks = torch.cat([torch.tensor(prompt, device=toks.device).expand(toks.shape[0], -1), toks], dim=1)
+            toks = torch.cat([torch.tensor(self._resolved(prompts, langs), device=toks.device, dtype=toks.dtype), toks], dim=1)
         return toks if feats.is_cuda else toks.cpu()
 
-    def _generate_seek_loop(self, feats, prompt, max_length, pad, return_prompt):
+    def _generate_seek_loop(self, feats, prompts, max_length, pad, return_prompt):
         tsb = self.generation_config.no_timestamps_token_id + 1
         B = feats.shape[0]
         x = feats.to(self.device).float()
         seek = [0] * B
         segs = [[] for _ in range(B)]
+        prompts = list(prompts)       # a row's detection slot is resolved on its first pass; the remainders reuse that prompt
         while any(s < N_FRAMES for s in seek):
             active = [i for i in range(B) if seek[i] < N_FRAMES]
             nframes = [min(N_FRAMES - seek[i], N_FRAMES) for i in active]
@@ -829,7 +1024,10 @@ class B200WhisperForConditionalGeneration:
             toks_l, lens_l = [], []
             for s0 in range(0, len(active), self.max_batch):
                 enc = self.encode(chunk[s0:s0 + self.max_batch])
-                t, l = self.decode(enc, prompt, max_length, True)
+                rows = active[s0:s0 + self.max_batch]
+                t, l, lg = self.decode_rows(enc, [prompts[i] for i in rows], max_length, True)
+                for i, p in zip(rows, self._resolved([prompts[i] for i in rows], lg.tolist())):
+                    prompts[i] = p
                 toks_l.append(t)
                 lens_l.append(l)
             toks = torch.cat(toks_l).cpu().numpy()
@@ -846,7 +1044,7 @@ class B200WhisperForConditionalGeneration:
         for i, r in enumerate(rows):
             out[i, :len(r)] = torch.from_numpy(r.astype(np.int64))
         if return_prompt:
-            out = torch.cat([torch.tensor(prompt).expand(B, -1), out], dim=1)
+            out = torch.cat([torch.tensor(prompts, dtype=out.dtype), out], dim=1)
         return out.to(feats.device) if feats.is_cuda else out
 
     # forward() (training) is out of scope

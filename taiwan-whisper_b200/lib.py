@@ -22,6 +22,7 @@ EXPORTS = [
     "tw_debug_absorbed_attention", "tw_pipeline_enable", "tw_pipeline_resize", "tw_pipeline_info", "tw_pipeline_stage_ms", "tw_pipeline_encode", "tw_pipeline_encode_at", "tw_pipeline_decode",
     "tw_debug_select_steps", "tw_debug_kv_append", "tw_debug_self_attention_step", "tw_debug_decode_attention_step",
     "tw_debug_layernorm", "tw_debug_cross_kv", "tw_debug_read_stage1", "tw_debug_decode_taps", "tw_debug_decoder_logits_taps",
+    "tw_decode_greedy_rows", "tw_transcribe_host_rows", "tw_pipeline_decode_rows", "tw_debug_select_steps_rows", "tw_detect_language",
 ]
 
 
@@ -39,6 +40,14 @@ class Rules(C.Structure):
                 ("begin_suppress", C.POINTER(C.c_int32)), ("n_begin_suppress", C.c_int32),
                 ("eos", C.c_int32), ("pad", C.c_int32), ("timestamp_begin", C.c_int32),
                 ("no_timestamps", C.c_int32), ("max_initial_timestamp_index", C.c_int32)]
+
+
+class PromptRows(C.Structure):
+    _fields_ = [("prompts", C.POINTER(C.c_int32)), ("lang_ids", C.POINTER(C.c_int32)), ("n_lang", C.c_int32),
+                ("out_lang", C.c_void_p)]
+
+
+PROMPT_DETECT = -1       # at prompt index 1: detect the row's language there
 
 
 class TwError(RuntimeError):
@@ -112,6 +121,13 @@ def load_library() -> C.CDLL:
     lib.tw_pipeline_encode.argtypes = [vp, vp, vp, C.c_int, C.c_int]
     lib.tw_pipeline_encode_at.argtypes = [vp, vp, vp, C.c_int, C.c_int, C.c_int]
     lib.tw_pipeline_decode.argtypes = [vp, C.c_int, C.c_int, C.POINTER(i32), C.c_int, C.POINTER(Rules), C.c_int, vp, vp]
+    rows = C.POINTER(PromptRows)
+    lib.tw_decode_greedy_rows.argtypes = [vp, vp, C.c_int, rows, C.c_int, C.POINTER(Rules), C.c_int, vp, vp, vp, vp, C.c_int, vp]
+    lib.tw_transcribe_host_rows.argtypes = [vp, vp, vp, C.c_int, rows, C.c_int, C.POINTER(Rules), C.c_int, vp, vp, vp]
+    lib.tw_pipeline_decode_rows.argtypes = [vp, C.c_int, C.c_int, rows, C.c_int, C.POINTER(Rules), C.c_int, vp, vp]
+    lib.tw_debug_select_steps_rows.argtypes = [vp, vp, i64, C.c_int, rows, C.c_int, C.POINTER(Rules), C.c_int, C.POINTER(i32), vp,
+                                               vp, C.c_int, vp, vp, vp, vp, vp]
+    lib.tw_detect_language.argtypes = [vp, vp, C.c_int, C.POINTER(i32), C.c_int, vp, vp]
     _lib = lib
     return lib
 
@@ -150,6 +166,19 @@ class Context:
 
     def launch_count(self) -> int:
         return int(self.lib.tw_launch_count(self.handle))
+
+
+def make_prompt_rows(prompts, lang_ids=None, out_lang=None):
+    """Returns (PromptRows struct, keepalive, P) from per-row prompt lists of one length (PROMPT_DETECT at index 1 = detect);
+    out_lang: address of the [B] int32 buffer for the languages, or None."""
+    P = len(prompts[0])
+    if any(len(p) != P for p in prompts):
+        raise ValueError("every row's prompt must have the same length")
+    flat = (C.c_int32 * (len(prompts) * P))(*[int(t) for p in prompts for t in p])
+    langs = (C.c_int32 * max(1, len(lang_ids or ())))(*[int(t) for t in (lang_ids or ())])
+    r = PromptRows(C.cast(flat, C.POINTER(C.c_int32)), C.cast(langs, C.POINTER(C.c_int32)) if lang_ids else None,
+                   len(lang_ids or ()), out_lang)
+    return r, (flat, langs), P
 
 
 def make_rules(suppress, begin_suppress, eos, pad, timestamp_begin, no_timestamps, max_initial_ts):

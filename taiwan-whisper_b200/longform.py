@@ -190,7 +190,7 @@ def stitch_windows_timestamps(outputs, timestamp_begin: int, special_ids=(), tim
     return chunks
 
 
-def transcribe_longform(model, pcm: torch.Tensor, *, language: str = "zh", task: str = "transcribe", max_length: int = 448,
+def transcribe_longform(model, pcm: torch.Tensor, *, language: Optional[str] = "zh", task: str = "transcribe", max_length: int = 448,
                         return_timestamps: bool = True, batch_size: Optional[int] = None, chunk_len: int = N_SAMPLES,
                         stride_left: Optional[int] = None, stride_right: Optional[int] = None, special_ids=(), merge: int = 1):
     """Config 5 end to end for one recording (1-D int16 / float32 CUDA tensor): zero-copy windowing + log-mel
@@ -199,7 +199,8 @@ def transcribe_longform(model, pcm: torch.Tensor, *, language: str = "zh", task:
     256-375 (preprocess_batch -> forward -> postprocess) with the windows batched `batch_size` (<= model.max_batch) at a
     time.  `merge` > 1 sends the windows through the encoder `batch_size` at a time and decodes `merge` such batches together
     (as many as fit model.max_batch): a decode step streams the decoder weights and runs its chain of small kernels once whatever
-    the row count (bench.py --workload longform: 561 -> 1088 audio-s/s with 5 x 32 windows per decode); per window nothing changes."""
+    the row count (bench.py --workload longform: 561 -> 1088 audio-s/s with 5 x 32 windows per decode); per window nothing changes.
+    language=None detects the language of every window on its own (in the first step of its decode), as HF does per chunk."""
     feats, strides = chunked_log_mel(pcm, model.shape.n_mel, chunk_len, stride_left, stride_right)
     bs = min(int(batch_size or model.max_batch), model.max_batch)
     gc = model.generation_config
@@ -208,10 +209,11 @@ def transcribe_longform(model, pcm: torch.Tensor, *, language: str = "zh", task:
     rows: List[List[int]] = []
     G = max(1, min(int(merge), model.max_batch // bs))
     if G > 1:
-        prompt = model._init_tokens(language, task, return_timestamps)
         for g0 in range(0, feats.shape[0], bs * G):
             encs = [model.encode(feats[b0:b0 + bs]) for b0 in range(g0, min(g0 + bs * G, feats.shape[0]), bs)]
-            toks, lens = model.decode(encs[0] if len(encs) == 1 else torch.cat(encs), prompt, max_length, return_timestamps)
+            enc = encs[0] if len(encs) == 1 else torch.cat(encs)
+            prompts = model._row_prompts(language, task, return_timestamps, enc.shape[0])
+            toks, lens, _ = model.decode_rows(enc, prompts, max_length, return_timestamps)
             toks, lens = toks.cpu().numpy(), lens.cpu().numpy()
             for r, n in zip(toks, lens):
                 r = r[:int(n)].tolist()

@@ -32,7 +32,7 @@ class Segment(NamedTuple):
 
 
 class TranscriptionInfo(NamedTuple):
-    language: str
+    language: Optional[str]      # None: every window's language was detected on its own
     duration: float
     n_windows: int
 
@@ -85,10 +85,11 @@ def save_transcription_to_csv(transcriptions: Iterable, output_csv: str):
 
 class B200BatchedInferencePipeline:
     """`pipeline.transcribe(audio=..., task="transcribe", log_progress=..., batch_size=...) -> (segments, info)` with
-    `segment.start / .end / .text`, as the reference calls it (ref: pseudo-labelling/initial_inference.py:36-45)."""
+    `segment.start / .end / .text`, as the reference calls it (ref: pseudo-labelling/initial_inference.py:36-45).
+    language=None (here and in transcribe) detects the language of every window on its own, as HF does per chunk."""
 
     def __init__(self, model, tokenizer=None, decode_fn: Optional[Callable[[List[int]], str]] = None, chunk_length: int = 30,
-                 language: str = "zh", use_vad_model: bool = False, max_length: int = 448):
+                 language: Optional[str] = "zh", use_vad_model: bool = False, max_length: int = 448):
         if use_vad_model:
             raise NotImplementedError("the Silero VAD model is third-party; this pipeline chunks by fixed windows")
         if not (1 <= chunk_length <= 30):
